@@ -31,6 +31,10 @@ style line (every rank a full batch of its own) next to it.
            DESIGN.md §4); E still counts every edge of the lattice, as the reference evaluates them.
 `cpu_baseline` = the oracle (a C restatement of vibrato's Rust path; the Rust toolchain is absent) timed with the
            reference's benchmark protocol body on one host thread, bounded sample.
+
+--dump-outputs DIR writes what the last timed step of `value` returned (the device-resident entry point's token
+offsets and token records) as DIR/<name>.npy, so that two builds can be compared output for output on the same
+seeded inputs; see dump_outputs() for the files.
 """
 import argparse
 import json
@@ -167,6 +171,60 @@ def make_inputs(cfg, rank, need_matrix, seed_rank=0):
     utf8, off = synth.make_corpus(sd, cfg["batch"], seed=20260923 + 2 + 1000 * seed_rank, **kw)
     log(f"[rank {rank}] corpus {cfg['batch']} sentences, {len(utf8) / 1e6:.1f} MB: {time.time() - t:.1f}s")
     return sd, user_csv, utf8, off
+
+
+def device_to_host(ptr, nbytes):
+    """Copies nbytes of device memory at ptr (a pointer the library returned) into a numpy uint8 array."""
+    import torch
+
+    class View:
+        __cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 3}
+
+    if nbytes == 0:
+        return np.zeros(0, dtype=np.uint8)
+    return torch.as_tensor(View(), device="cuda").cpu().numpy()
+
+
+DUMP_SEED = 20261017
+# Every token covers at least one input byte, so the sample holds at most 900 000 tokens (43.2 MB as 6 float64 fields);
+# with the per-sentence counts (<= 16 MB) and the sample's index and offsets (<= 1.1 MB) the files stay under 64 MB.
+DUMP_SAMPLE_INPUT_BYTES = 900_000
+DUMP_SAMPLE_MAX_SENTENCES = 65536
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, tok_off, tokens, off):
+    """Writes one step's result as float64 / float32 .npy files (every value is exact in its type):
+
+    tokens_per_sentence  float32 [n_sent]   token count of every sentence of the batch (left out above 4 M sentences)
+    sentence_index       float64 [S]        a fixed sample of sentences (seeded from DUMP_SEED and the input lengths only)
+    tok_offsets          float64 [S + 1]    where each sampled sentence's tokens start in the arrays below
+    <field>              float64 [T]        start_char, end_char, start_byte, end_byte, word_idx, total_cost of the
+                                            sampled sentences' tokens, in sentence order
+    """
+    import vibrato_b200 as vb
+    n = len(tok_off) - 1
+    tok_off = tok_off.astype(np.int64)
+    files = {}
+    if n <= 4_000_000:
+        files["tokens_per_sentence"] = np.diff(tok_off).astype(np.float32)
+    order = np.random.default_rng(DUMP_SEED).permutation(n)
+    in_bytes = np.cumsum(np.diff(off.astype(np.int64))[order])
+    k = min(int(np.searchsorted(in_bytes, DUMP_SAMPLE_INPUT_BYTES, side="right")), DUMP_SAMPLE_MAX_SENTENCES)
+    idx = np.sort(order[:k])
+    counts = tok_off[idx + 1] - tok_off[idx]
+    sample_off = np.concatenate([[0], np.cumsum(counts)])
+    rows = np.arange(sample_off[-1]) - np.repeat(sample_off[:-1] - tok_off[idx], counts)
+    files["sentence_index"] = idx.astype(np.float64)
+    files["tok_offsets"] = sample_off.astype(np.float64)
+    for name in vb.TOKEN_DTYPE.names:
+        files[name] = tokens[name][rows].astype(np.float64)
+    total = sum(a.nbytes for a in files.values())
+    assert total <= DUMP_MAX_BYTES, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in files.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"outputs of the last timed step: {len(files)} arrays, {total / 1e6:.1f} MB -> {out_dir}")
 
 
 def workload_config(cfg_id, cfg):
@@ -370,9 +428,13 @@ def run_ours(args, cfg_id, cfg, rank, world, local_rank):
 
     dev_ms, _ = timed(lambda: step_device(mine), 0, W)  # warm-up only
     stage_acc[:] = 0
-    dev_ms, _ = timed(dev_step, args.steps, 0)
+    dev_ms, last = timed(dev_step, args.steps, 0)
     check(lib().vbt_last_launch_count(h, C.byref(nl)))
     launches_per_step = nl.value
+    if args.dump_outputs:  # fetched now: the next call on this tokenizer reuses the result buffers
+        p_off, p_tok, n_last = last
+        last_tok_off = device_to_host(p_off, (mine.n + 1) * 8).view("<u8")
+        last_tokens = device_to_host(p_tok, n_last * vb.TOKEN_DTYPE.itemsize).view(vb.TOKEN_DTYPE)
 
     # --- e2e: host buffers in, host tokens out (pinned, then pageable) ----------------------------------
     e2e_ms, nt_host = timed(lambda: step_host(mine), args.steps, 2)
@@ -493,6 +555,8 @@ def run_ours(args, cfg_id, cfg, rank, world, local_rank):
             line["gathered"] = gathered
         if weak:
             line["weak"] = weak
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_tok_off, last_tokens, off)
         emit(line)
     lib().vbt_tokenizer_free(h)
     if dist:
@@ -508,13 +572,19 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=int(os.environ.get("VBT_BENCH_CONFIG", "3")), choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the token offsets / records of the last timed step as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if os.environ.get("VBT_BENCH_BATCH"):  # developer override (smoke runs)
         cfg["batch"] = int(os.environ["VBT_BENCH_BATCH"])
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs writes the GPU arm's result on one GPU (--impl ours, --gpus 1)")
     if args.impl == "reference":
         run_reference(args, args.config, cfg, rank, world)
     else:
