@@ -25,7 +25,7 @@ for ign in (0, 1):
         tok.set_option("chunk_sentences", chunk)
         res = tok.tokenize_batch(sents)
         print("ignore_space", ign, "lanes", lanes, "smem", smem, "chunk", chunk, "tokens", res.n_tokens, flush=True)
-# round 2: every Viterbi kernel (0 = k_viterbi, 1 = k_viterbi2 pruned, 2 = its unpruned twin), the retry paths
+# every K3 instantiation the matrix connector can take (0 = 64-bit-address lookup, 1 = pruned, 2 = unpruned twin)
 for kernel in (0, 1, 2):
     tok = vb.Tokenizer.new(d).ignore_space(True)
     tok.set_option("viterbi_kernel", kernel)

@@ -114,8 +114,8 @@ def test_fixture_batch_matches_oracle(golden, ignore_space, max_grouping):
 @pytest.mark.parametrize("lanes,sort,chunk", [(4, 1, 0), (8, 0, 1000), (16, 1, 777), (32, 0, 0), (8, 1, 2500), (16, 0, 0),
                                               (32, 1, 1500)])
 def test_viterbi_lane_layouts_match_oracle(lanes, sort, chunk):
-    """Every lanes-per-sentence layout of k_viterbi, both sentence orders and the chunked (pipelined)
-    host path give identical tokens."""
+    """Every lanes-per-sentence layout of k_viterbi2, both sentence orders and the chunked (pipelined)
+    host path give identical tokens and counters."""
     sd = synth.make_dictionary("synth-small")
     d = vb.SystemDictionaryBuilder.from_readers(sd.lex_csv, sd.matrix, sd.char_def, sd.unk_def)
     od = vo.OracleDictionary(sd.lex_csv, sd.matrix, sd.char_def, sd.unk_def)

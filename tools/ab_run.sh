@@ -1,5 +1,5 @@
 #!/bin/bash
-# Developer tool (GPU box): timing of the k_viterbi variants built by tools/build_variants.sh (one process each).
+# Developer tool (GPU box): timing of the k_viterbi2 variants built by tools/build_variants.sh (one process each).
 #   tools/ab_run.sh "variant[:layout]" ...     -> gpurun_out/ab.txt
 cd "$(dirname "$0")/.."
 R=$PWD/vibrato_b200

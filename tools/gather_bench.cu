@@ -1,7 +1,7 @@
 // Microbenchmark: how many random 2-byte lookups per second can one B200 sustain on a
 // unidic-sized connection matrix (15626 x 15388 i16 = 459 MiB) when the ids follow the same
 // Zipf(1.0) law as the synthetic dictionary, (a) with ids in random order, (b) frequency-sorted?
-// This is the practical ceiling for k_viterbi's dominant access pattern.
+// This is the practical ceiling for K3's dominant access pattern.
 //   nvcc -O3 -gencode arch=compute_100a,code=sm_100a -o tools/gather_bench tools/gather_bench.cu
 #include <cuda_runtime.h>
 

@@ -1,4 +1,4 @@
-"""Lattice statistics that decide k_viterbi's design (run on the CPU with the analysis build of the oracle).
+"""Lattice statistics that decide K3's design (run on the CPU with the analysis build of the oracle).
 
 For the synthetic workloads of bench.py: how many distinct right ids a lattice row has, how many distinct left
 ids the candidates of a position have (the gain of de-duplicating connection-cost lookups), and how many

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Developer tool: times the device-resident step for several k_viterbi layouts on one dictionary.
+"""Developer tool: times the device-resident step for several k_viterbi2 lane layouts on one dictionary.
     python tools/sweep.py [dict] [batch] [fixed_len]"""
 import ctypes as C
 import os

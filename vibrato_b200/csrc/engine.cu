@@ -143,12 +143,12 @@ __global__ void k_add_value(unsigned long long* tok_off, uint32_t n_plus_1, unsi
 
 struct Workspace {  // every per-(chunk of a)-batch device array; two of them let consecutive chunks overlap
     DevBuf n_slots, slot_off, eos, n_tok, code_sys, code_usr, cinfo, groupable, byte_pos, info, info_ex, ends_cnt,
-        ends_meta, cand, ends_hot, ends_cold, scan_tmp, stats, iota, sort_keys, order;
+        ends_meta, cand, ends_hot, ends_cold, scan_tmp, iota, sort_keys, order;
     cudaStream_t stream = nullptr;
     void release() {
         for (DevBuf* b : {&n_slots, &slot_off, &eos, &n_tok, &code_sys, &code_usr, &cinfo, &groupable, &byte_pos, &info,
-                          &info_ex, &ends_cnt, &ends_meta, &cand, &ends_hot, &ends_cold, &scan_tmp, &stats, &iota,
-                          &sort_keys, &order})
+                          &info_ex, &ends_cnt, &ends_meta, &cand, &ends_hot, &ends_cold, &scan_tmp, &iota, &sort_keys,
+                          &order})
             b->release();
     }
 };
@@ -846,7 +846,6 @@ class EngineImpl final : public Engine {
         w.info_ex.ensure(ms * 8, 1.25);
         w.ends_cnt.ensure(ms * 4, 1.25);
         w.ends_meta.ensure(ms * 8, 1.25);
-        if (counting_) w.stats.ensure(ms * 16, 1.25);
         size_t want_cand = std::max<size_t>(1 << 16, size_t(double(n_bytes) * cand_per_byte_) + 4096);
         want_cand = std::min<size_t>(want_cand, 0xFFFFFFF0ull);
         w.cand.ensure(want_cand * 16);
@@ -977,14 +976,14 @@ class EngineImpl final : public Engine {
         launch_decode(dv_, b, st);
         CK(cudaEventRecord(o.ev[3], st));
         launch_candidates(dv_, b, max_slots, st);
-        if (counting_) {
-            launch_candidate_stats(dv_, b, max_slots, w.stats.as<uint4>(), st);
-            ++o.launches;
-        }
         CK(cudaEventRecord(o.ev[4], st));
         exclusive_scan(w, b.ends_cnt, RowMetaOut{b.ends_meta}, size_t(max_slots) + 1);
         CK(cudaEventRecord(o.ev[5], st));
-        o.launches += launch_viterbi(dv_, b, counting_ ? w.stats.as<uint4>() : nullptr, lanes_, viterbi_kernel_, st);
+        o.launches += launch_viterbi(dv_, b, lanes_, viterbi_kernel_, st);
+        if (b.counters || b.lid_count) {
+            launch_count_lattice(dv_, b, st);
+            ++o.launches;
+        }
         CK(cudaEventRecord(o.ev[6], st));
         launch_backtrack_count(b, st);
         CK(cudaEventRecord(o.ev[7], st));

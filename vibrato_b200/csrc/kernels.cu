@@ -3,7 +3,9 @@
 //   K1a count_chars     warp / sentence   UTF-8 validation + character count
 //   K1b decode          warp / sentence   code points -> CharInfo, trie codes, c2b, groupable
 //   K2  candidates      thread / char     common-prefix walks (user, system) + unknown words
-//   K3  viterbi         warp / sentence   left-to-right min-plus DP over the lattice + EOS
+//   K3  viterbi2        G lanes / sentence left-to-right min-plus DP over the lattice + EOS
+//       count_lattice   thread / sentence counted runs only: SURVEY.md §8(d) counters and connection-id counts,
+//                                         read off the finished lattice
 //   K4a backtrack_count thread / sentence length of the best path
 //   K4b backtrack_write thread / sentence token records, in sentence order
 //
@@ -12,14 +14,6 @@
 #include "kernels.cuh"
 
 #include <climits>
-
-// Minimum resident blocks per SM asked of ptxas for k_viterbi (128 threads each): 16 -> 32 registers,
-// 64 warps/SM.  Measured on B200 (synth-unidic, 1 M sentences): 10 blocks 14.2 ms, 12 -> 13.6 ms, 16 -> 12.0 ms
-// (r01c); with the slot-absolute loop state of r01e the 32-register build no longer spills (12 blocks: 12.0 ms,
-// 16 blocks: 11.1 ms).  The counting and Raw/Dual instantiations are not on the timed path and get 64 registers.
-#ifndef VBT_K3_MIN_BLOCKS
-#define VBT_K3_MIN_BLOCKS 16
-#endif
 
 // A batch whose byte offsets k_count_chars refused is not touched by any later kernel: the sizes derived from
 // the offsets (slots, workspace bounds) cannot be trusted.
@@ -354,7 +348,7 @@ __device__ __forceinline__ uint32_t gen_unknown(const DictView& d, uint32_t sw, 
 }
 
 __global__ void __launch_bounds__(256) k_candidates(DictView d, Batch b) {
-    constexpr bool COUNT = false;  // M/T/P/W are produced by k_candidate_stats in counted runs
+    constexpr bool COUNT = false;  // M/T/P/W are produced by k_count_lattice in counted runs
     const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t lane = threadIdx.x & 31;
     // A rejected batch (see VBT_STAND_DOWN_IF_REJECTED) leaves every thread out of range.  The flag word is read
@@ -491,66 +485,26 @@ __global__ void __launch_bounds__(256) k_candidates(DictView d, Batch b) {
     (void)st;
 }
 
-// Side array for counted runs: per slot {M, T, P, W} so that k_viterbi can sum them over the
-// positions the reference actually visits.  Filled by a second, counting-only kernel.
-__global__ void __launch_bounds__(256) k_candidate_stats(DictView d, Batch b, uint4* stats) {
-    VBT_STAND_DOWN_IF_REJECTED(b);
-    const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot >= b.slot_off[b.n_sent]) return;
-    uint32_t g0 = b.groupable[slot];
-    uint4 out = make_uint4(0, 0, 0, 0);
-    if (g0 != 0) {
-        uint32_t sw = slot, ci0 = b.cinfo[slot];
-        if (ci_cate(ci0) & d.space_mask) sw = slot + g0;
-        uint32_t g = b.groupable[sw];
-        if (g != 0) {
-            WalkStats st{0, 0, 0, 0, 0};
-            uint32_t cu = 0;
-            if (d.usr_table)
-                cu = walk_lexicon<false, true>(d.usr_nodes, d.usr_num_nodes, d.usr_post, b.code_usr, b.groupable, sw,
-                                               nullptr, nullptr, st);
-            uint32_t cs = walk_lexicon<false, true>(d.sys_nodes, d.sys_num_nodes, d.sys_post, b.code_sys, b.groupable,
-                                                    sw, nullptr, nullptr, st);
-            uint32_t ck = gen_unknown<false>(d, sw, b.cinfo[sw], g, (cu + cs) != 0, nullptr, nullptr);
-            out = make_uint4(st.m, st.t, st.p, st.w + ck);
-            out.x |= st.walks << 24;  // <= 2 walks; M stays far below 2^24 per position
-        }
-    }
-    stats[slot] = out;
-}
-
 // ---------------------------------------------------------------------------------------------
 // K3: Tokenizer::build_lattice_inner (tokenizer.rs:94-139) + Lattice::insert_node / search_min_node /
 //     insert_eos (lattice.rs:85-151).
 //
-// G lanes per sentence (32 / G sentences per warp, walking their positions in lockstep): lane j of a
-// group owns candidate j of the current start position, the group's predecessors {cost, right} are
-// staged in registers and broadcast with width-G shuffles.  The typical position has ~7 candidates
-// and ~8 predecessors, so G = 8 keeps most lanes busy where one warp per sentence left 3/4 idle.
+// G lanes per sentence (32 / G sentences per warp, walking their start positions in lockstep, one position after
+// the other), built around what the r01f profile showed to be the limits — warp-instruction issue and the LSU data
+// pipe of the L1 (shuffles, spills and gathers all queue there):
+//   * per position the candidates of the warp's sentences are dealt to the 32 lanes as one pool, lane = candidate;
+//     the typical position has ~7 candidates and ~8 predecessors;
+//   * the predecessors {cost, right} of a position are staged once in shared memory and read back two at a time
+//     with one LDS.128 (a broadcast inside the group) instead of two SHFL per predecessor;
+//   * the gather address is one multiply-add on a per-candidate column pointer (the matrix is stored transposed);
+//   * no state is carried across positions except three slot numbers: nothing spills at 32 registers;
+//   * exact lower-bound pruning (PRUNE): every candidate record carries lb = min over ALL right ids of
+//     M[right][left], so a predecessor with cost + lb > best-so-far cannot reach the minimum, not even tie it,
+//     and its gather is skipped.  Predecessors are still visited in row order with `<=`, so the LAST minimal one
+//     wins exactly as in Lattice::search_min_node (lattice.rs:129-151).  The bound arithmetic assumes that no i32
+//     addition wraps: batches holding a sentence longer than kPruneMaxChars characters take the unpruned path,
+//     which keeps the reference's wrapping adds.
 // ---------------------------------------------------------------------------------------------
-
-// Candidate header of one start position as {cand_ptr, cand_cnt, skip, flags}; the last two live in a side array
-// that only the few positions with a skipped space run or the trailing flag ever touch.
-__device__ __forceinline__ uint4 load_info(const Batch& b, uint32_t slot) {
-    const uint2 i8 = b.info[slot];
-    uint4 r = make_uint4(i8.x, i8.y & ~kInfoSpecial, 0, 0);
-    if (i8.y & kInfoSpecial) {
-        const uint2 ex = b.info_ex[slot];
-        r.z = ex.x;
-        r.w = ex.y;
-    }
-    return r;
-}
-
-// Build-time switches of k_viterbi, kept for A/B builds (tools/build_variants.sh; profiles/r01e_k3_variants_ab.md):
-// VBT_K3_PF_DIST = how many candidates ahead one lane per group hints into L1 (0 = no hint), VBT_K3_PIPE = fetch a
-// position's row metadata and candidate header one position early.
-#ifndef VBT_K3_PF_DIST
-#define VBT_K3_PF_DIST 8
-#endif
-#ifndef VBT_K3_PIPE
-#define VBT_K3_PIPE 1
-#endif
 
 // ConnectorCost::cost(right_id, left_id) for one fixed left id (one candidate).
 template <int CONN>
@@ -613,269 +567,16 @@ struct ConnRow<2> {  // DualConnector::cost (dual_connector.rs:269-280): reduced
     }
 };
 
-template <int G, bool COUNT, int CONN>
-__global__ void __launch_bounds__(128, (CONN == 0 && !COUNT) ? VBT_K3_MIN_BLOCKS : 8) k_viterbi(DictView d, Batch b, const uint4* __restrict__ stats) {
-    VBT_STAND_DOWN_IF_REJECTED(b);
-    constexpr uint32_t SPW = 32 / G;  // sentences per warp
-    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t sub = lane / G, gl = lane % G;
-    const uint32_t sidx = warp * SPW + sub;
-    const bool has_sentence = sidx < b.n_sent;
-    unsigned long long cntE = 0, cntN = 2, cM = 0, cT = 0, cP = 0, cW = 0, cWalks = 0;
-
-    // Loop state is kept slot-absolute (current slot, the slot whose row EOS connects to, first slot after a
-    // skipped space run) so that nothing but these three words lives across the gather loop; the sentence
-    // index, its base slot and its length are looked up again where the sweep ends.
-    uint32_t slot = 0, slot_end = 0;
-    if (has_sentence) {
-        const uint32_t s = b.order ? b.order[sidx] : sidx;
-        slot = b.slot_off[s];
-        slot_end = b.slot_off[s + 1] - 1;
-        if (gl == 0) {
-            if (slot == slot_end) {  // Worker::tokenize returns early on an empty sentence (worker.rs:50-52)
-                b.eos[s] = make_uint4(kNone, 0, 0, 0);
-            } else {  // Lattice::insert_bos (lattice.rs:72-83): right_id 0, cost 0
-                const uint32_t eo = b.ends_meta[slot].x;
-                b.ends_hot[eo] = make_int2(0, 0);
-                b.ends_cold[eo] = make_uint4(kNone, kNone, kNone, 0);
-                b.ends_meta[slot].y = eo + 1;
-            }
-        }
-    }
-    __syncwarp();
-
-    uint32_t skip_slot = slot;
-#if VBT_K3_PIPE
-    // Row metadata and candidate header of a position are fetched one position early, so that its candidates and
-    // predecessors can be requested as soon as the position starts (one round trip less on the chain).
-    uint2 m_cur = make_uint2(0, 0);
-    uint4 info_cur = make_uint4(0, 0, 0, 0);
-    if (slot < slot_end) {
-        m_cur = b.ends_meta[slot];
-        info_cur = load_info(b, slot);
-    }
-    const uint32_t group_mask = G == 32 ? kFull : (((1u << (G & 31)) - 1u) << (sub * G));
-#endif
-    while (__any_sync(kFull, slot < slot_end)) {
-        const bool active = slot < slot_end;
-        uint32_t K = 0, eo = 0;
-        uint4 info = make_uint4(0, 0, 0, 0);
-#if VBT_K3_PIPE
-        if (active) {
-            eo = m_cur.x;
-            K = m_cur.y - m_cur.x;
-            info = info_cur;
-        }
-        // A fill count read this early misses the nodes this very position appends to the next row: k_fix
-        // carries the count the group itself wrote there.
-        uint2 m_nx = make_uint2(0, 0);
-        uint4 info_nx = make_uint4(0, 0, 0, 0);
-        uint32_t k_fix = 0;
-        if (active && slot + 1 < slot_end) {
-            m_nx = b.ends_meta[slot + 1];
-            info_nx = load_info(b, slot + 1);
-        }
-#else
-        if (active) {  // two independent loads, one round trip
-            const uint2 m = b.ends_meta[slot];
-            info = load_info(b, slot);
-            eo = m.x;
-            K = m.y - m.x;
-        }
-#endif
-        // positions inside a skipped space run are never start_node; K == 0: has_previous_node fails
-        bool visit = active && slot >= skip_slot && K != 0;  // (lattice.rs:155-157, tokenizer.rs:110-114)
-        if (visit && (info.w & kInfoTrailing)) {  // tokenizer.rs:128-130: EOS starts here, the sweep ends
-            slot_end = slot;
-            visit = false;
-        }
-        if (visit && info.z) skip_slot = slot + info.z + 1;  // next start_node = start_word + 1 (tokenizer.rs:134-135)
-        const uint32_t ncand = visit ? info.y : 0;
-        if (COUNT && stats && visit && gl == 0) {
-            uint4 stv = stats[slot];
-            cWalks += stv.x >> 24;
-            cM += stv.x & 0xFFFFFFu;
-            cT += stv.y;
-            cP += stv.z;
-            cW += stv.w;
-            cntE += (unsigned long long)K * ncand;
-            cntN += ncand;
-        }
-#if VBT_K3_PF_DIST
-        // K2 hands out the candidate pool in position order, so the candidates of the positions ahead follow
-        // this position's; K2 wrote them long ago (evicted from L2), pull the line ahead while this position works
-        if (visit && gl == 0 && info.x + ncand + VBT_K3_PF_DIST < b.cand_cap) {
-            const uint4* nx = b.cand + info.x + ncand + VBT_K3_PF_DIST;
-#if VBT_K3_PF_L2
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(nx));
-#else
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(nx));
-#endif
-        }
-#endif
-        const uint32_t max_cand = __reduce_max_sync(kFull, ncand);
-        // first chunk of predecessors: independent of the candidates, so issue it alongside their load
-        int2 pr_first = make_int2(0, 0);
-        if (visit && gl < K) pr_first = b.ends_hot[eo + gl];
-        for (uint32_t c0 = 0; c0 < max_cand; c0 += G) {
-            const bool valid = c0 + gl < ncand;
-            uint4 cd = make_uint4(0, 0, 0, 0);
-            uint32_t fill = 0;
-            if (valid) {
-                cd = b.cand[info.x + c0 + gl];
-                // row metadata of the node's end position: independent of the minimum search, fetch now
-                const uint2 me = b.ends_meta[cd.w];
-                fill = me.y;  // next free entry of that row (absolute)
-            }
-            const uint32_t left = cd.x & 0xFFFFu, right = cd.x >> 16;
-            const ConnRow<CONN> conn(d, left);
-            // Lattice::add_connid_counts (lattice.rs:170-176): one (left, pred.right) edge per predecessor
-            if (COUNT && b.lid_count && valid) atomicAdd(&b.lid_count[left], (unsigned long long)K);
-            // Lattice::search_min_node (lattice.rs:129-151): `<=` keeps the LAST minimum
-            int32_t best = INT32_MAX;
-            uint32_t bestk = 0;
-            const uint32_t Kv = valid ? K : 0;
-            const uint32_t max_k = __reduce_max_sync(kFull, Kv);
-            for (uint32_t k0 = 0; k0 < max_k; k0 += G) {
-                int2 pr = pr_first;
-                if (k0 != 0) {
-                    pr = make_int2(0, 0);
-                    if (k0 + gl < K) pr = b.ends_hot[eo + k0 + gl];
-                }
-                if (COUNT && b.rid_count && c0 == 0 && k0 + gl < K && ncand)
-                    atomicAdd(&b.rid_count[uint32_t(pr.y)], (unsigned long long)ncand);
-                const uint32_t kc = min(uint32_t(G), max_k - k0);
-#pragma unroll 8
-                for (uint32_t kk = 0; kk < kc; ++kk) {
-                    int32_t pc = __shfl_sync(kFull, pr.x, kk, G);
-                    uint32_t prr = uint32_t(__shfl_sync(kFull, pr.y, kk, G));
-                    if (k0 + kk < Kv) {
-                        // MatrixConnector::cost (matrix_connector.rs:79-85,121-124); i32 wrapping add
-                        int32_t v = int32_t(uint32_t(pc) + uint32_t(conn.cost(d, prr)));
-                        if (v <= best) {
-                            best = v;
-                            bestk = k0 + kk;
-                        }
-                    }
-                }
-            }
-            // Lattice::insert_node (lattice.rs:103-127): push into ends[end_word] in candidate order.
-            // End slots of different sentences never coincide, so one warp-wide match suffices.
-            const uint32_t vmask = __ballot_sync(kFull, valid);
-            if (valid) {
-                const uint32_t peers = __match_any_sync(vmask, cd.w);
-                const uint32_t rank = __popc(peers & lanemask_lt());
-                const uint32_t idx = fill + rank;
-                const int32_t cost = int32_t(uint32_t(best) + uint32_t(int32_t(int16_t(cd.y & 0xFFFFu))));
-                b.ends_hot[idx] = make_int2(cost, int32_t(right));
-                // lattice.rs:144 keeps the predecessor index as u16
-                b.ends_cold[idx] = make_uint4(slot, eo + (bestk & 0xFFFFu), cd.z, uint32_t(cost));
-                if (rank == 0) b.ends_meta[cd.w].y = fill + __popc(peers);
-#if VBT_K3_PIPE
-                if (rank == 0 && cd.w == slot + 1) k_fix = fill + __popc(peers);
-#endif
-            }
-            __syncwarp();
-        }
-#if VBT_K3_PIPE
-        k_fix = __reduce_max_sync(group_mask, k_fix);  // fills only grow: the last chunk's count is the largest
-        m_cur = make_uint2(m_nx.x, max(m_nx.y, k_fix));
-        info_cur = info_nx;
-#endif
-        if (slot < slot_end) ++slot;
-    }
-
-    // Lattice::insert_eos (lattice.rs:85-101): left_id 0, no word cost; lanes of the group = predecessors
-    {
-        const uint32_t s = has_sentence ? (b.order ? b.order[sidx] : sidx) : 0;
-        const uint32_t base = has_sentence ? b.slot_off[s] : 0;
-        const uint32_t n = has_sentence ? b.slot_off[s + 1] - 1 - base : 0;
-        const uint32_t eos_start = slot_end - base;  // n, or the start of the trailing space run
-        uint32_t K = 0, eo = 0;
-        if (n > 0) {
-            const uint2 m = b.ends_meta[slot_end];
-            eo = m.x;
-            K = m.y - m.x;
-        }
-        // minimise the signed 64-bit key (cost << 32 | ~index): smallest cost, then the LARGEST index
-        // among ties — the `<=` rule of search_min_node
-        long long bestkey = LLONG_MAX;
-        const ConnRow<CONN> conn_eos(d, 0);  // BOS_EOS_CONNECTION_ID (common.rs:18)
-        const uint32_t max_k = __reduce_max_sync(kFull, K);
-        for (uint32_t k0 = 0; k0 < max_k; k0 += G) {
-            long long key = LLONG_MAX;
-            if (k0 + gl < K) {
-                int2 pr = b.ends_hot[eo + k0 + gl];
-                int32_t v = int32_t(uint32_t(pr.x) + uint32_t(conn_eos.cost(d, uint32_t(pr.y))));
-                key = (long long)(((unsigned long long)uint32_t(v) << 32) | (unsigned long long)(~(k0 + gl)));
-            }
-#pragma unroll
-            for (int o = G / 2; o > 0; o >>= 1) key = min(key, __shfl_xor_sync(kFull, key, o, G));
-            bestkey = min(bestkey, key);
-        }
-        if (COUNT) cntE += K;
-        if (COUNT && b.lid_count && n > 0) {  // lattice.rs:178-181: the EOS edges are counted over ends[len_char]
-            const uint2 ml = b.ends_meta[base + n];
-            const uint32_t nl = ml.y - ml.x;
-            for (uint32_t k = gl; k < nl; k += G) atomicAdd(&b.rid_count[uint32_t(b.ends_hot[ml.x + k].y)], 1ull);
-            if (gl == 0 && nl) atomicAdd(&b.lid_count[0], (unsigned long long)nl);
-        }
-        if (n > 0 && gl == 0) {
-            const bool none = K == 0;
-            const uint32_t bestk = (~uint32_t(bestkey)) & 0xFFFFu;  // lattice.rs:144 `i as u16`
-            b.eos[s] = make_uint4(none ? kNone : eo + bestk, eos_start, uint32_t(int32_t(bestkey >> 32)), 0);
-        }
-        if (COUNT && b.counters && n > 0 && gl == 0) {
-            atomicAdd(&b.counters[kCntE], cntE);
-            atomicAdd(&b.counters[kCntN], cntN);
-            atomicAdd(&b.counters[kCntM], cM);
-            atomicAdd(&b.counters[kCntT], cT);
-            atomicAdd(&b.counters[kCntP], cP);
-            atomicAdd(&b.counters[kCntW], cW);
-            atomicAdd(&b.counters[kCntWalks], cWalks);
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// K3, second design (round 2).  Same mapping as k_viterbi (G lanes per sentence, lane = candidate, sequential over
-// start positions), rebuilt around what the r01f profile showed to be the limits — warp-instruction issue and the
-// LSU data pipe of the L1 (shuffles, spills and gathers all queue there):
-//   * the predecessors {cost, right} of a position are staged once in shared memory and read back two at a time
-//     with one LDS.128 (a broadcast inside the group) instead of two SHFL per predecessor;
-//   * the gather address is one multiply-add on a per-candidate column pointer (the matrix is stored transposed);
-//   * no state is carried across positions except three slot numbers: nothing spills at 32 registers;
-//   * exact lower-bound pruning (PRUNE): every candidate record carries lb = min over ALL right ids of
-//     M[right][left], so a predecessor with cost + lb > best-so-far cannot reach the minimum, not even tie it,
-//     and its gather is skipped.  Predecessors are still visited in row order with `<=`, so the LAST minimal one
-//     wins exactly as in Lattice::search_min_node (lattice.rs:129-151).  The bound arithmetic assumes that no i32
-//     addition wraps: batches holding a sentence longer than kPruneMaxChars characters take the unpruned path,
-//     which keeps the reference's wrapping adds.
-// ---------------------------------------------------------------------------------------------
-
 #ifndef VBT_K3V2_WARPS
 #define VBT_K3V2_WARPS 4  // warps per block of k_viterbi2
 #endif
 #ifndef VBT_K3V2_MIN_BLOCKS
 #define VBT_K3V2_MIN_BLOCKS (64 / VBT_K3V2_WARPS)  // 64 warps per SM = 32 registers per thread
 #endif
-#ifndef VBT_K3V2_BATCH
-#define VBT_K3V2_BATCH 2  // predecessors whose gathers are issued together (2 or 4); 4 spills at 32 registers
-#endif
-#ifndef VBT_K3V2_FIRST
-#define VBT_K3V2_FIRST 0  // 1 = the first predecessor of a row is evaluated alone, ahead of the batches
-#endif
 #ifndef VBT_K3V2_PF_DIST
 #define VBT_K3V2_PF_DIST 8
 #endif
 
-#ifndef VBT_K3V2_BULK
-#define VBT_K3V2_BULK 0
-#endif
-#if VBT_K3V2_BULK
-constexpr uint32_t kCandWin = 8;  // candidates per sentence in the bulk-copied window
-#endif
 constexpr int kPredCap = 32;                             // predecessors staged per pass
 constexpr int32_t kPredSentinel = INT32_MAX - 70000;     // + any i16 stays below INT32_MAX and above every real best
 
@@ -906,7 +607,7 @@ struct ConnCol<0> {
             : "r"(right), "r"(stride2), "r"(colbase), "r"(hi));
         return m;
     }
-    // U predecessors of Lattice::search_min_node, staged at shared address `pp` as {cost, right} pairs.  Phase 1
+    // Two predecessors of Lattice::search_min_node, staged at shared address `pp` as {cost, right} pairs.  Phase 1
     // tests every one of them (PRUNE: cost + lb <= best, lb = cost_word >> 16; otherwise: its address lies below
     // `plim`, the end of this lane's row) and issues the surviving 2-byte gathers together; phase 2 folds them in
     // row order with `<=`, so the LAST minimum wins.  A bound that is one batch old is still a bound: `best` only
@@ -922,16 +623,6 @@ struct ConnCol<0> {
 #define VBT_V2_HEAD "{\n\t.reg .pred q;\n\t.reg .s32 t, lb;\n\t.reg .u32 k;\n\t"
 #define VBT_V2_OPERANDS \
     : "+r"(best), "+r"(besttok) : "r"(pp), "r"(PRUNE ? cost_word : plim), "r"(stride2), "r"(colbase), "r"(hi)
-    template <bool PRUNE>
-    __device__ __forceinline__ void batch1(uint32_t pp, uint32_t cost_word, uint32_t plim, int32_t& best,
-                                           uint32_t& besttok) const {
-        if (PRUNE)
-            asm volatile(VBT_V2_HEAD VBT_V2_DECL(0) "ld.shared.v2.b32 {c0, r0}, [%2];\n\tshr.s32 lb, %3, 16;\n\t"  //
-                         VBT_V2_TEST_PRUNE(0) VBT_V2_LOAD(0) VBT_V2_FOLD(0) "}" VBT_V2_OPERANDS);
-        else
-            asm volatile(VBT_V2_HEAD VBT_V2_DECL(0) "ld.shared.v2.b32 {c0, r0}, [%2];\n\t"  //
-                         VBT_V2_TEST_PLAIN(0) VBT_V2_LOAD(0) VBT_V2_FOLD(0) "}" VBT_V2_OPERANDS);
-    }
     // `zero` is a run-time zero the compiler cannot see through: the first fold reads m0 | (m1 & zero) = m0, one
     // LOP3 that needs BOTH gathers, so the two loads are issued back to back (left alone, ptxas at 32 registers
     // sinks the second load below the first fold and the two round trips serialise).
@@ -950,30 +641,15 @@ struct ConnCol<0> {
                          VBT_V2_TEST_PLAIN(0) VBT_V2_TEST_PLAIN(1) VBT_V2_LOAD(0) VBT_V2_LOAD(1)  //
                          VBT_V2_FOLD0_JOIN(1) VBT_V2_FOLD(1) "}" VBT_V2_OPERANDS, "r"(zero));
     }
-    template <bool PRUNE>
-    __device__ __forceinline__ void batch4(uint32_t pp, uint32_t cost_word, uint32_t plim, int32_t& best,
-                                           uint32_t& besttok) const {
-#define VBT_V2_LDS4 "ld.shared.v4.b32 {c0, r0, c1, r1}, [%2];\n\tld.shared.v4.b32 {c2, r2, c3, r3}, [%2+16];\n\t"
-        if (PRUNE)
-            asm volatile(VBT_V2_HEAD VBT_V2_DECL(0) VBT_V2_DECL(1) VBT_V2_DECL(2) VBT_V2_DECL(3) VBT_V2_LDS4 "shr.s32 lb, %3, 16;\n\t"
-                         VBT_V2_TEST_PRUNE(0) VBT_V2_TEST_PRUNE(1) VBT_V2_TEST_PRUNE(2) VBT_V2_TEST_PRUNE(3)  //
-                         VBT_V2_LOAD(0) VBT_V2_LOAD(1) VBT_V2_LOAD(2) VBT_V2_LOAD(3)                          //
-                         "lop3.b32 m1, m1, m2, m3, 0xF0;\n\t" /* = m1, after all three arrived */                     //
-                         VBT_V2_FOLD0_JOIN(1) VBT_V2_FOLD(1) VBT_V2_FOLD(2) VBT_V2_FOLD(3) "}" VBT_V2_OPERANDS, "r"(zero));
-        else
-            asm volatile(VBT_V2_HEAD VBT_V2_DECL(0) VBT_V2_DECL(1) VBT_V2_DECL(2) VBT_V2_DECL(3) VBT_V2_LDS4
-                         VBT_V2_TEST_PLAIN(0) VBT_V2_TEST_PLAIN(1) VBT_V2_TEST_PLAIN(2) VBT_V2_TEST_PLAIN(3)  //
-                         VBT_V2_LOAD(0) VBT_V2_LOAD(1) VBT_V2_LOAD(2) VBT_V2_LOAD(3)                          //
-                         "lop3.b32 m1, m1, m2, m3, 0xF0;\n\t"                                                         //
-                         VBT_V2_FOLD0_JOIN(1) VBT_V2_FOLD(1) VBT_V2_FOLD(2) VBT_V2_FOLD(3) "}" VBT_V2_OPERANDS, "r"(zero));
-    }
 };
 
-// Raw / Dual connectors: plain C++ over ConnRow::cost, same interface.
+// Raw / Dual connectors, and the matrix with 64-bit addresses (CONN 3: a matrix that crosses a 4 GiB address
+// boundary, and the `viterbi_kernel = 0` check of that path): plain C++ over ConnRow::cost, same interface.
 template <int CONN>
-struct ConnCol : ConnRow<CONN> {
+struct ConnCol : ConnRow<CONN == 3 ? 0 : CONN> {
+    using Row = ConnRow<CONN == 3 ? 0 : CONN>;
     const DictView& dv;
-    __device__ __forceinline__ ConnCol(const DictView& d, uint32_t left) : ConnRow<CONN>(d, left), dv(d) {}
+    __device__ __forceinline__ ConnCol(const DictView& d, uint32_t left) : Row(d, left), dv(d) {}
     template <bool PRUNE>
     __device__ __forceinline__ void batch1(uint32_t pp, uint32_t, uint32_t plim, int32_t& best, uint32_t& besttok) const {
         if (pp < plim) {
@@ -991,11 +667,6 @@ struct ConnCol : ConnRow<CONN> {
 #pragma unroll
         for (int i = 0; i < 2; ++i) batch1<PRUNE>(pp + 8 * i, cw, plim, best, besttok);
     }
-    template <bool PRUNE>
-    __device__ __forceinline__ void batch4(uint32_t pp, uint32_t cw, uint32_t plim, int32_t& best, uint32_t& besttok) const {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) batch1<PRUNE>(pp + 8 * i, cw, plim, best, besttok);
-    }
 };
 
 // Shared-memory window of one warp of k_viterbi2: a staging row per sentence ({cost, right} of the predecessors, up
@@ -1008,12 +679,6 @@ struct V2Shared {
     int2 rows[SPW][kPredCap + 4];
     uint4 desc[SPW];
     uint32_t cnt[8];
-#if VBT_K3V2_BULK
-    // candidate windows: the first kCandWin candidates of every sentence's NEXT position, fetched one position ahead
-    // by a bulk asynchronous copy (cp.async.bulk, completion counted on an mbarrier); two buffers alternate
-    uint4 cwin[2][SPW][kCandWin];
-    unsigned long long mbar[2];
-#endif
 };
 
 template <int G, int CONN, bool PRUNE, bool SPACE>
@@ -1024,28 +689,6 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t gl = lane % G, sub = lane / G;
     const uint32_t sidx = ((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * SPW + sub;
-#if VBT_K3V2_BULK
-    constexpr uint32_t kWinOff = kCntOff + 32, kWinBytes = SPW * kCandWin * 16, kBarOff = kWinOff + 2 * kWinBytes;
-    // issues the bulk copy of the first candidates of position `at` into window `buf` (leaders only) and arrives on
-    // that window's barrier; a position without candidates (or past the end) arrives without a copy
-    auto prefetch_candidates = [&](uint32_t at, bool in_sentence, uint32_t buf) {
-        uint32_t nb = 0;
-        uint2 inx = make_uint2(0, 0);
-        if (in_sentence) inx = b.info[at];
-        nb = min(inx.y & ~kInfoSpecial, kCandWin) * 16u;
-        const uint32_t bar = sw + kBarOff + buf * 8u;
-        if (nb) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(nb) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             sw + kWinOff + buf * kWinBytes + sub * (kCandWin * 16u)),
-                         "l"(b.cand + inx.x), "r"(nb), "r"(bar)
-                         : "memory");
-        } else {
-            asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-        }
-    };
-#endif
 
     uint32_t slot = 0, slot_end = 0;
     if (sidx < b.n_sent) {
@@ -1064,23 +707,9 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
         }
     }
     __syncwarp();
-#if VBT_K3V2_BULK
-    if (lane == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(sw + kBarOff), "r"(SPW) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(sw + kBarOff + 8u), "r"(SPW) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    uint32_t it = 0;  // iteration of the lockstep walk: window it & 1, barrier parity (it >> 1) & 1
-    if (gl == 0) prefetch_candidates(slot, slot < slot_end, 0);
-#endif
 
     uint32_t skip_slot = slot;
     while (__any_sync(kFull, slot < slot_end)) {
-#if VBT_K3V2_BULK
-        // the candidates of the NEXT position start travelling now, into the other window
-        if (gl == 0) prefetch_candidates(slot + 1, slot + 1 < slot_end, (it + 1) & 1);
-#endif
         uint32_t K = 0, eo = 0, cptr = 0, ncand = 0;
         if (slot < slot_end) {  // two independent loads, one round trip
             const uint2 m = b.ends_meta[slot];
@@ -1125,11 +754,10 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
         // global -> shared without a register or a scoreboard entry in between) so that it overlaps the loads of
         // the candidates below; the copies are awaited right before the first batch.  Rows are 8-byte aligned only,
         // which rules out the 16-byte granular bulk copies (cp.async.bulk).
-        constexpr uint32_t B = VBT_K3V2_BATCH, F = VBT_K3V2_FIRST;
         const bool one_pass = max_k <= uint32_t(kPredCap);
         if (one_pass && total) {
-            const uint32_t n_stage = F + ((max_k - F + (B - 1u)) & ~(B - 1u));
-            const uint32_t own = sw + sub * kRowBytes + 8u * F;
+            const uint32_t n_stage = (max_k + 1u) & ~1u;
+            const uint32_t own = sw + sub * kRowBytes;
 #pragma unroll 1
             for (uint32_t k = gl; k < n_stage; k += G) {
                 if (k < K)
@@ -1139,15 +767,6 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
             }
         }
         __syncwarp();
-#if VBT_K3V2_BULK
-        {  // this position's window: every lane waits every iteration, which also keeps the barrier phases in step
-            const uint32_t bar = sw + kBarOff + (it & 1u) * 8u, parity = (it >> 1) & 1u;
-            asm volatile(
-                "{\n\t.reg .pred p;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(bar),
-                "r"(parity)
-                : "memory");
-        }
-#endif
         for (uint32_t q0 = 0; q0 < total; q0 += 32) {
             const uint32_t q = q0 + lane;
             const bool valid = q < total;
@@ -1172,14 +791,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
             uint4 cd = make_uint4(0, 0, 0, 0);
             uint32_t nxt = 0;
             if (valid) {
-#if VBT_K3V2_BULK
-                if (q - before < kCandWin)  // arrived with the window (awaited above)
-                    asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
-                                 : "=r"(cd.x), "=r"(cd.y), "=r"(cd.z), "=r"(cd.w)
-                                 : "r"(sw + kWinOff + (it & 1u) * kWinBytes + (s2 * kCandWin + (q - before)) * 16u));
-                else
-#endif
-                    cd = b.cand[ds.x + (q - before)];
+                cd = b.cand[ds.x + (q - before)];
                 nxt = b.ends_meta[cd.w].y;  // next free entry of the row the node ends in: independent of the search
             }
             const ConnCol<CONN> conn(d, cd.x & 0xFFFFu);
@@ -1189,10 +801,9 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
 #pragma unroll 1
             for (uint32_t k0 = 0; k0 < max_k; k0 += kPredCap) {
                 // This pass covers predecessors [k0, k0 + kc) of every row, staged by the row's own group and padded
-                // with sentinels to whole batches.  With VBT_K3V2_FIRST the first one is evaluated alone (its total is
-                // the bound the batches start from) and sits one entry in, so that the batches stay 16-byte aligned.
+                // with sentinels to whole batches.
                 const uint32_t kc = min(uint32_t(kPredCap), max_k - k0);
-                const uint32_t n_stage = F + ((kc - F + (B - 1u)) & ~(B - 1u));
+                const uint32_t n_stage = (kc + 1u) & ~1u;
                 if (one_pass) {
                     if (q0 == 0) {  // the copies started above have had the candidates' round trip to arrive
                         asm volatile("cp.async.wait_all;" ::: "memory");
@@ -1200,7 +811,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
                     }
                 } else {  // rows longer than kPredCap: pass after pass, staged synchronously
                     __syncwarp();
-                    const uint32_t own = sw + sub * kRowBytes + 8u * F;
+                    const uint32_t own = sw + sub * kRowBytes;
 #pragma unroll 1
                     for (uint32_t k = gl; k < n_stage; k += G) {
                         int2 pr = make_int2(kPredSentinel, 0);
@@ -1210,18 +821,12 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
                     __syncwarp();
                 }
                 // the shared address of a predecessor doubles as its token: index = k0 + (token - row) / 8
-                const uint32_t row = sw + s2 * kRowBytes + 8u * F;
+                const uint32_t row = sw + s2 * kRowBytes;
                 const uint32_t plim = row + (valid ? min(ds.w - min(ds.w, k0), kc) : 0u) * 8u;  // end of this lane's row
                 uint32_t besttok = kNone;
-                if (F) conn.template batch1<PRUNE>(row, cd.y, plim, best, besttok);
                 const uint32_t pend = row + n_stage * 8u;
 #pragma unroll 1
-                for (uint32_t pp = row + 8u * F; pp < pend; pp += 8u * B) {
-                    if (B == 2)
-                        conn.template batch2<PRUNE>(pp, cd.y, plim, best, besttok);
-                    else
-                        conn.template batch4<PRUNE>(pp, cd.y, plim, best, besttok);
-                }
+                for (uint32_t pp = row; pp < pend; pp += 16u) conn.template batch2<PRUNE>(pp, cd.y, plim, best, besttok);
                 if (besttok != kNone) bestk = k0 + ((besttok - row) >> 3);
             }
             // Lattice::insert_node (lattice.rs:103-127): push into ends[end_word] in candidate order.
@@ -1239,9 +844,6 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
             __syncwarp();
         }
         if (slot < slot_end) ++slot;
-#if VBT_K3V2_BULK
-        ++it;
-#endif
     }
 
     // Lattice::insert_eos (lattice.rs:85-101): left_id 0, no word cost; lanes of the group = predecessors
@@ -1292,6 +894,93 @@ __global__ void __launch_bounds__(32 * VBT_K3V2_WARPS, CONN == 0 ? VBT_K3V2_MIN_
     __shared__ __align__(16) V2Shared<G> s_warp[VBT_K3V2_WARPS];
     const uint32_t sp = uint32_t(__cvta_generic_to_shared(&s_warp[threadIdx.x >> 5]));
     viterbi2_sweep<G, CONN, PRUNE, SPACE>(d, b, sp);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Counted runs only: the SURVEY.md §8(d) counters M, T, P, W, walks, E, N and Lattice::add_connid_counts
+// (lattice.rs:170-181), read off the finished lattice after K3 and before K4a reuses `ends_meta`.  A thread walks
+// the start positions of its sentence as K3 did; a row's size after K3 is the K that K3 saw at that position, since
+// only earlier positions append to it.
+// ---------------------------------------------------------------------------------------------
+
+// Candidate header of one start position as {cand_ptr, cand_cnt, skip, flags}; the last two live in a side array
+// that only the few positions with a skipped space run or the trailing flag ever touch.
+__device__ __forceinline__ uint4 load_info(const Batch& b, uint32_t slot) {
+    const uint2 i8 = b.info[slot];
+    uint4 r = make_uint4(i8.x, i8.y & ~kInfoSpecial, 0, 0);
+    if (i8.y & kInfoSpecial) {
+        const uint2 ex = b.info_ex[slot];
+        r.z = ex.x;
+        r.w = ex.y;
+    }
+    return r;
+}
+
+__global__ void __launch_bounds__(256) k_count_lattice(DictView d, Batch b) {
+    VBT_STAND_DOWN_IF_REJECTED(b);
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= b.n_sent) return;
+    const uint32_t base = b.slot_off[s], n = b.slot_off[s + 1] - 1 - base;
+    if (n == 0) return;  // Worker::tokenize returns early on an empty sentence (worker.rs:50-52)
+    unsigned long long cE = 0, cN = 2, cM = 0, cT = 0, cP = 0, cW = 0, cWalks = 0;
+    uint32_t slot_end = base + n, skip_slot = base;
+    for (uint32_t slot = base; slot < slot_end; ++slot) {
+        const uint2 m = b.ends_meta[slot];
+        const uint32_t K = m.y - m.x;
+        // positions inside a skipped space run are never start_node; K == 0: has_previous_node fails
+        if (slot < skip_slot || K == 0) continue;  // (lattice.rs:155-157, tokenizer.rs:110-114)
+        const uint4 info = load_info(b, slot);
+        if (info.w & kInfoTrailing) {  // tokenizer.rs:128-130: EOS starts here
+            slot_end = slot;
+            break;
+        }
+        if (info.z) skip_slot = slot + info.z + 1;  // next start_node = start_word + 1 (tokenizer.rs:134-135)
+        const uint32_t ncand = info.y;
+        cE += (unsigned long long)K * ncand;
+        cN += ncand;
+        if (b.counters) {  // k_candidates' walks from start_word again, counting (also where ncand == 0)
+            const uint32_t sw = slot + info.z;
+            WalkStats st{0, 0, 0, 0, 0};
+            uint32_t cu = 0;
+            if (d.usr_table)
+                cu = walk_lexicon<false, true>(d.usr_nodes, d.usr_num_nodes, d.usr_post, b.code_usr, b.groupable, sw,
+                                               nullptr, nullptr, st);
+            const uint32_t cs = walk_lexicon<false, true>(d.sys_nodes, d.sys_num_nodes, d.sys_post, b.code_sys,
+                                                          b.groupable, sw, nullptr, nullptr, st);
+            const uint32_t ck =
+                gen_unknown<false>(d, sw, b.cinfo[sw], b.groupable[sw], (cu + cs) != 0, nullptr, nullptr);
+            cM += st.m;
+            cT += st.t;
+            cP += st.p;
+            cW += st.w + ck;
+            cWalks += st.walks;
+        }
+        if (b.lid_count) {  // Lattice::add_connid_counts (lattice.rs:170-176): one (left, pred.right) edge per predecessor
+            for (uint32_t c = 0; c < ncand; ++c)
+                atomicAdd(&b.lid_count[b.cand[info.x + c].x & 0xFFFFu], (unsigned long long)K);
+            if (ncand)
+                for (uint32_t k = 0; k < K; ++k)
+                    atomicAdd(&b.rid_count[uint32_t(b.ends_hot[m.x + k].y)], (unsigned long long)ncand);
+        }
+    }
+    // Lattice::insert_eos (lattice.rs:85-101) connects the row of slot_end
+    const uint2 me = b.ends_meta[slot_end];
+    cE += me.y - me.x;
+    if (b.lid_count) {  // lattice.rs:178-181: the EOS edges are counted over ends[len_char]
+        const uint2 ml = b.ends_meta[base + n];
+        const uint32_t nl = ml.y - ml.x;
+        for (uint32_t k = 0; k < nl; ++k) atomicAdd(&b.rid_count[uint32_t(b.ends_hot[ml.x + k].y)], 1ull);
+        if (nl) atomicAdd(&b.lid_count[0], (unsigned long long)nl);
+    }
+    if (b.counters) {
+        atomicAdd(&b.counters[kCntE], cE);
+        atomicAdd(&b.counters[kCntN], cN);
+        atomicAdd(&b.counters[kCntM], cM);
+        atomicAdd(&b.counters[kCntT], cT);
+        atomicAdd(&b.counters[kCntP], cP);
+        atomicAdd(&b.counters[kCntW], cW);
+        atomicAdd(&b.counters[kCntWalks], cWalks);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1553,71 +1242,50 @@ void launch_candidates(const DictView& d, const Batch& b, uint32_t max_slots, cu
     k_candidates<<<blocks, 256, 0, st>>>(d, b);
 }
 
-void launch_candidate_stats(const DictView& d, const Batch& b, uint32_t max_slots, uint4* stats, cudaStream_t st) {
-    if (!max_slots) return;
-    uint32_t blocks = (max_slots + 255) / 256;
-    k_candidate_stats<<<blocks, 256, 0, st>>>(d, b, stats);
-}
-
 template <int G>
-static int launch_viterbi_g(const DictView& d, const Batch& b, const uint4* stats, int kernel, cudaStream_t st) {
-    const uint32_t per_block = 4 * (32 / G);  // 4 warps per block
+static int launch_viterbi_g(const DictView& d, const Batch& b, int kernel, cudaStream_t st) {
+    const bool space = d.space_mask != 0;
+    const uint32_t per_block = VBT_K3V2_WARPS * (32 / G);
     const uint32_t blocks = (b.n_sent + per_block - 1) / per_block;
-    const bool counted = stats || b.lid_count;
-    // k_viterbi2's matrix lookups assume a matrix inside one 4 GiB window (the engine arranges that when it can)
-    if (!counted && kernel != 0 && (d.connector_kind != 0 || d.matrix_window)) {
-        const bool space = d.space_mask != 0;
-        const uint32_t per_block2 = VBT_K3V2_WARPS * (32 / G);
-        const uint32_t blocks2 = (b.n_sent + per_block2 - 1) / per_block2;
-#define VBT_LAUNCH_V2(CONN, PRUNE, TWIN)                                        \
-    do {                                                                        \
-        if (space)                                                              \
-            k_viterbi2<G, CONN, PRUNE, true, TWIN><<<blocks2, 32 * VBT_K3V2_WARPS, 0, st>>>(d, b);  \
-        else                                                                    \
-            k_viterbi2<G, CONN, PRUNE, false, TWIN><<<blocks2, 32 * VBT_K3V2_WARPS, 0, st>>>(d, b); \
+#define VBT_LAUNCH_V2(CONN, PRUNE, TWIN)                                                          \
+    do {                                                                                          \
+        if (space)                                                                                \
+            k_viterbi2<G, CONN, PRUNE, true, TWIN><<<blocks, 32 * VBT_K3V2_WARPS, 0, st>>>(d, b); \
+        else                                                                                      \
+            k_viterbi2<G, CONN, PRUNE, false, TWIN><<<blocks, 32 * VBT_K3V2_WARPS, 0, st>>>(d, b); \
     } while (0)
-        if (d.connector_kind == 1) {
-            VBT_LAUNCH_V2(1, false, false);
-        } else if (d.connector_kind == 2) {
-            VBT_LAUNCH_V2(2, false, false);
-        } else if (kernel == 1) {  // the pruned kernel and its twin for batches with very long sentences
-            VBT_LAUNCH_V2(0, true, true);
-            VBT_LAUNCH_V2(0, false, true);
-        } else {
-            VBT_LAUNCH_V2(0, false, false);
-        }
-#undef VBT_LAUNCH_V2
-        return (d.connector_kind == 0 && kernel == 1) ? 2 : 1;
-    }
+    int launched = 1;
     if (d.connector_kind == 1) {
-        if (counted)
-            k_viterbi<G, true, 1><<<blocks, 128, 0, st>>>(d, b, stats);
-        else
-            k_viterbi<G, false, 1><<<blocks, 128, 0, st>>>(d, b, stats);
+        VBT_LAUNCH_V2(1, false, false);
     } else if (d.connector_kind == 2) {
-        if (counted)
-            k_viterbi<G, true, 2><<<blocks, 128, 0, st>>>(d, b, stats);
-        else
-            k_viterbi<G, false, 2><<<blocks, 128, 0, st>>>(d, b, stats);
-    } else if (counted) {
-        k_viterbi<G, true, 0><<<blocks, 128, 0, st>>>(d, b, stats);
+        VBT_LAUNCH_V2(2, false, false);
+    } else if (kernel == 0 || !d.matrix_window) {  // ConnCol<0> needs the matrix inside one 4 GiB window
+        VBT_LAUNCH_V2(3, false, false);
+    } else if (kernel == 1) {  // the pruned kernel and its twin for batches with very long sentences
+        VBT_LAUNCH_V2(0, true, true);
+        VBT_LAUNCH_V2(0, false, true);
+        launched = 2;
     } else {
-        k_viterbi<G, false, 0><<<blocks, 128, 0, st>>>(d, b, stats);
+        VBT_LAUNCH_V2(0, false, false);
     }
-    return 1;
+#undef VBT_LAUNCH_V2
+    return launched;
 }
 
-int launch_viterbi(const DictView& d, const Batch& b, const uint4* stats, int lanes_per_sentence, int kernel,
-                   cudaStream_t st) {
+int launch_viterbi(const DictView& d, const Batch& b, int lanes_per_sentence, int kernel, cudaStream_t st) {
     if (!b.n_sent) return 0;
     switch (lanes_per_sentence) {
-        case 4: return launch_viterbi_g<4>(d, b, stats, kernel, st);
-        case 8: return launch_viterbi_g<8>(d, b, stats, kernel, st);
-        case 32: return launch_viterbi_g<32>(d, b, stats, kernel, st);
-        default: return launch_viterbi_g<16>(d, b, stats, kernel, st);
+        case 4: return launch_viterbi_g<4>(d, b, kernel, st);
+        case 8: return launch_viterbi_g<8>(d, b, kernel, st);
+        case 32: return launch_viterbi_g<32>(d, b, kernel, st);
+        default: return launch_viterbi_g<16>(d, b, kernel, st);
     }
 }
 
+void launch_count_lattice(const DictView& d, const Batch& b, cudaStream_t st) {
+    if (!b.n_sent) return;
+    k_count_lattice<<<(b.n_sent + 255) / 256, 256, 0, st>>>(d, b);
+}
 
 void launch_backtrack_count(const Batch& b, cudaStream_t st) {
     if (!b.n_sent) return;

@@ -138,14 +138,14 @@ void launch_format_write(const DictView& d, const FormatArgs& f, cudaStream_t st
 void launch_count_chars(const Batch& b, cudaStream_t st);
 void launch_decode(const DictView& d, const Batch& b, cudaStream_t st);
 void launch_candidates(const DictView& d, const Batch& b, uint32_t max_slots, cudaStream_t st);
-// Counted runs only: per-slot {M | walks << 24, T, P, W} of SURVEY.md §8(d), summed by K3 over visited positions.
-void launch_candidate_stats(const DictView& d, const Batch& b, uint32_t max_slots, uint4* stats, cudaStream_t st);
-// lanes_per_sentence in {4, 8, 16, 32}: how many lanes of a warp cooperate on one sentence.
-// stats != nullptr or b.lid_count != nullptr selects the counting instantiation.
-// kernel: 0 = k_viterbi (round 1), 1 = k_viterbi2 (predecessors staged in shared memory, lower-bound pruning),
-// 2 = k_viterbi2 without pruning.  Counted runs always use k_viterbi.  Returns the number of kernels launched.
-int launch_viterbi(const DictView& d, const Batch& b, const uint4* stats, int lanes_per_sentence, int kernel,
-                   cudaStream_t st);
+// K3 = k_viterbi2.  lanes_per_sentence in {4, 8, 16, 32}: how many lanes of a warp cooperate on one sentence.
+// kernel (matrix connector only): 1 = lower-bound pruning, with its unpruned twin for batches with very long
+// sentences; 2 = unpruned; 0 = the unpruned 64-bit-address lookup that a matrix crossing a 4 GiB address boundary
+// takes anyway.  Returns the number of kernels launched.
+int launch_viterbi(const DictView& d, const Batch& b, int lanes_per_sentence, int kernel, cudaStream_t st);
+// Counted runs only (b.counters or b.lid_count): the SURVEY.md §8(d) counters M, T, P, W, walks, E, N and the
+// connection-id counts, read off the lattice K3 left.  Runs between K3 and launch_backtrack_count.
+void launch_count_lattice(const DictView& d, const Batch& b, cudaStream_t st);
 void launch_backtrack_count(const Batch& b, cudaStream_t st);
 void launch_backtrack_write(const Batch& b, cudaStream_t st);
 
