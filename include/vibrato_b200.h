@@ -225,11 +225,9 @@ void vbt_host_free(void *p);
  * algorithmic-byte counters U,C,M,T,P,W,E,N,K of SURVEY.md §8(d) measured on the device. */
 /* Turns the device-side counters on or off (off by default: they cost an extra walk per position). */
 int32_t vbt_tokenizer_set_counting(vbt_tokenizer *t, int32_t on);
-/* Tuning knobs (results never change): "lanes_per_sentence" = 4|8|16|32 lanes of a warp per sentence in the
- * Viterbi kernel (default 8), "sort_by_length" = 0|1 (default 0: process sentences in input order),
- * "chunk_sentences" = sentences per chunk of the pipelined host path (default 262144, 0 = off),
- * "dual_stream" = 0|1 (default 0: chunks share one compute stream), "counting" = 0|1,
- * "connid_counting" = 0|1 (see vbt_connid_counts), "output_mode" = 0|1|2|3 (see vbt_result_text; default 0). */
+/* Tuning knobs (results never change): "chunk_sentences" = sentences per chunk of the pipelined host path
+ * (default 262144, 0 = off), "counting" = 0|1, "connid_counting" = 0|1 (see vbt_connid_counts),
+ * "output_mode" = 0|1|2|3 (see vbt_result_text; default 0). */
 int32_t vbt_tokenizer_set_option(vbt_tokenizer *t, const char *name, int64_t value);
 /* Worker::init_connid_counter / update_connid_counts / compute_connid_probs (worker.rs:77-103): switch
  * the option "connid_counting" on (this zeroes the counters), tokenise the corpus, then read the edge

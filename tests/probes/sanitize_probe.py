@@ -20,17 +20,17 @@ d.reset_user_lexicon_from_reader(r["user.csv"])
 sents = [c["input"] for c in g["tokenizer_cases"]] * 20 + ["X" * 300, "", "0123456789" * 40]
 for ign in (0, 1):
     tok = vb.Tokenizer.new(d).ignore_space(bool(ign)).max_grouping_len(24 if ign else 0)
-    for lanes, smem, chunk in ((16, 0, 0), (8, 0, 100), (32, 0, 64)):
-        tok.set_option("lanes_per_sentence", lanes)
+    for chunk in (0, 100, 64):
         tok.set_option("chunk_sentences", chunk)
         res = tok.tokenize_batch(sents)
-        print("ignore_space", ign, "lanes", lanes, "smem", smem, "chunk", chunk, "tokens", res.n_tokens, flush=True)
-# every K3 instantiation the matrix connector can take (0 = 64-bit-address lookup, 1 = pruned, 2 = unpruned twin)
-for kernel in (0, 1, 2):
+        print("ignore_space", ign, "chunk", chunk, "tokens", res.n_tokens, flush=True)
+# every K3 instantiation the matrix connector can take (0 = 64-bit-address lookup, 1 = pruned, and its unpruned twin
+# for a batch with a sentence of more than kPruneMaxChars characters)
+for kernel, extra in ((0, []), (1, []), (1, ["X" * 16001])):
     tok = vb.Tokenizer.new(d).ignore_space(True)
     tok.set_option("viterbi_kernel", kernel)
-    res = tok.tokenize_batch(sents)
-    print("viterbi_kernel", kernel, "tokens", res.n_tokens, flush=True)
+    res = tok.tokenize_batch(sents + extra)
+    print("viterbi_kernel", kernel, "long sentence", bool(extra), "tokens", res.n_tokens, flush=True)
 sd = synth.make_dictionary("synth-tiny")
 d2 = vb.SystemDictionaryBuilder.from_readers(sd.lex_csv, sd.matrix, sd.char_def, sd.unk_def)
 od = vo.OracleDictionary(sd.lex_csv, sd.matrix, sd.char_def, sd.unk_def)
@@ -82,9 +82,8 @@ print("device-resident + multi engine ok", flush=True)
 rows = "\n".join(f"a,1,1,{1000 - (i % 7)},h{i}" for i in range(600)) + "\nb,1,1,5,B\n"
 dl = vb.SystemDictionaryBuilder.from_readers(rows, "2 2\n0 0 0\n0 1 0\n1 0 0\n1 1 0\n", "DEFAULT 0 1 0\n", "DEFAULT,0,0,30000,*\n")
 ol = vo.OracleDictionary(rows, "2 2\n0 0 0\n0 1 0\n1 0 0\n1 1 0\n", "DEFAULT 0 1 0\n", "DEFAULT,0,0,30000,*\n")
-u8, o = vb.Tokenizer.pack(["abab", "a", "bba"] * 5)
-for kernel in (1, 2):
+for long in ([], ["b" * 16001]):  # pruned, then the unpruned twin
+    u8, o = vb.Tokenizer.pack(["abab", "a", "bba"] * 5 + long)
     t = vb.Tokenizer.new(dl)
-    t.set_option("viterbi_kernel", kernel)
     assert t.tokenize_batch(utf8=u8, byte_offsets=o).tokens.tobytes() == ol.tokenize_batch(u8, o)[1].tobytes()
 print("long rows ok", flush=True)

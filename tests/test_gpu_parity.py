@@ -111,11 +111,10 @@ def test_fixture_batch_matches_oracle(golden, ignore_space, max_grouping):
     np.testing.assert_array_equal(tok.last_counters(), cnt)
 
 
-@pytest.mark.parametrize("lanes,sort,chunk", [(4, 1, 0), (8, 0, 1000), (16, 1, 777), (32, 0, 0), (8, 1, 2500), (16, 0, 0),
-                                              (32, 1, 1500)])
-def test_viterbi_lane_layouts_match_oracle(lanes, sort, chunk):
-    """Every lanes-per-sentence layout of k_viterbi2, both sentence orders and the chunked (pipelined)
-    host path give identical tokens and counters."""
+@pytest.mark.parametrize("chunk", [0, 777, 1000, 1500, 2500, 4000, 5000])
+def test_chunked_host_path_matches_oracle(chunk):
+    """The whole-batch and the chunked (pipelined) host path give identical tokens and counters, from the smallest
+    chunks to a chunk size that leaves the 6005 sentences in one piece (5000)."""
     sd = synth.make_dictionary("synth-small")
     d = vb.SystemDictionaryBuilder.from_readers(sd.lex_csv, sd.matrix, sd.char_def, sd.unk_def)
     od = vo.OracleDictionary(sd.lex_csv, sd.matrix, sd.char_def, sd.unk_def)
@@ -127,10 +126,7 @@ def test_viterbi_lane_layouts_match_oracle(lanes, sort, chunk):
     utf8 = np.concatenate([utf8, u2])
     off = np.concatenate([off, o2[1:] + off[-1]])
     tok = vb.Tokenizer.new(d)
-    tok.set_option("lanes_per_sentence", lanes)
-    tok.set_option("sort_by_length", sort)
     tok.set_option("chunk_sentences", chunk)
-    tok.set_option("dual_stream", lanes == 8)
     tok.set_counting(True)
     res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
     tok_off, toks, cnt = od.tokenize_batch(utf8, off, n_threads=8, want_counters=True)
@@ -302,14 +298,12 @@ def test_many_prefix_hits_per_position():
     od = vo.OracleDictionary(lex, matrix, chardef, unk).set_user_csv(user)
     sents = ["a" * 40, "b" * 5 + "a" * 20 + "b" * 3, "ab" * 30, "bbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbbb", "a" * 14 + "z" + "a" * 3]
     utf8, off = vb.Tokenizer.pack(sents * 40)
-    for lanes in (8, 16, 32):
-        tok = vb.Tokenizer.new(d)
-        tok.set_option("lanes_per_sentence", lanes)
-        tok.set_counting(True)
-        res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
-        tok_off, toks, cnt = od.tokenize_batch(utf8, off, want_counters=True)
-        assert_batch_equal(res, tok_off, toks)
-        np.testing.assert_array_equal(tok.last_counters(), cnt)
+    tok = vb.Tokenizer.new(d)
+    tok.set_counting(True)
+    res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
+    tok_off, toks, cnt = od.tokenize_batch(utf8, off, want_counters=True)
+    assert_batch_equal(res, tok_off, toks)
+    np.testing.assert_array_equal(tok.last_counters(), cnt)
 
 
 def test_connid_counters_and_reordering(golden):
@@ -380,19 +374,17 @@ def test_raw_connector_dictionary_matches_oracle():
     d = vb.SystemDictionaryBuilder.from_readers_with_bigram_info(sd.lex_csv, right, left, cost, sd.char_def, sd.unk_def)
     od = vo.OracleDictionary(sd.lex_csv, (right, left, cost), sd.char_def, sd.unk_def)
     utf8, off = synth.make_corpus(sd, 5000, seed=8, log_uniform=(1, 200), unk_frac=0.1, space_frac=0.02)
-    for lanes in (8, 16, 32):
-        tok = vb.Tokenizer.new(d).ignore_space(True)
-        tok.set_option("lanes_per_sentence", lanes)
-        tok.set_counting(True)
-        tok.init_connid_counter()
-        res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
-        tok_off, toks, cnt = od.tokenize_batch(utf8, off, True, n_threads=8, want_counters=True)
-        assert_batch_equal(res, tok_off, toks)
-        np.testing.assert_array_equal(tok.last_counters(), cnt)
-        lid, rid = tok.connid_counts()
-        olid, orid = od.connid_counts(utf8, off, True, n_threads=8)
-        np.testing.assert_array_equal(lid, olid)
-        np.testing.assert_array_equal(rid, orid)
+    tok = vb.Tokenizer.new(d).ignore_space(True)
+    tok.set_counting(True)
+    tok.init_connid_counter()
+    res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
+    tok_off, toks, cnt = od.tokenize_batch(utf8, off, True, n_threads=8, want_counters=True)
+    assert_batch_equal(res, tok_off, toks)
+    np.testing.assert_array_equal(tok.last_counters(), cnt)
+    lid, rid = tok.connid_counts()
+    olid, orid = od.connid_counts(utf8, off, True, n_threads=8)
+    np.testing.assert_array_equal(lid, olid)
+    np.testing.assert_array_equal(rid, orid)
     d2 = vb.Dictionary.read(d.write())
     res2 = vb.Tokenizer.new(d2).ignore_space(True).tokenize_batch(utf8=utf8, byte_offsets=off)
     assert_batch_equal(res2, tok_off, toks)
@@ -409,18 +401,16 @@ def test_dual_connector_dictionary_matches_oracle():
     od = vo.OracleDictionary(sd.lex_csv, (right, left, cost), sd.char_def, sd.unk_def, dual_connector=True)
     utf8, off = synth.make_corpus(sd, 5000, seed=9, log_uniform=(1, 200), unk_frac=0.1, space_frac=0.02)
     tok_off, toks, cnt = od.tokenize_batch(utf8, off, True, n_threads=8, want_counters=True)
-    for lanes in (8, 16, 32):
-        tok = vb.Tokenizer.new(d).ignore_space(True)
-        tok.set_option("lanes_per_sentence", lanes)
-        tok.set_counting(True)
-        tok.init_connid_counter()
-        res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
-        assert_batch_equal(res, tok_off, toks)
-        np.testing.assert_array_equal(tok.last_counters(), cnt)
-        lid, rid = tok.connid_counts()
-        olid, orid = od.connid_counts(utf8, off, True, n_threads=8)
-        np.testing.assert_array_equal(lid, olid)
-        np.testing.assert_array_equal(rid, orid)
+    tok = vb.Tokenizer.new(d).ignore_space(True)
+    tok.set_counting(True)
+    tok.init_connid_counter()
+    res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
+    assert_batch_equal(res, tok_off, toks)
+    np.testing.assert_array_equal(tok.last_counters(), cnt)
+    lid, rid = tok.connid_counts()
+    olid, orid = od.connid_counts(utf8, off, True, n_threads=8)
+    np.testing.assert_array_equal(lid, olid)
+    np.testing.assert_array_equal(rid, orid)
     # the Raw connector over the same files stores the same cost function
     raw = build(sd.lex_csv, right, left, cost, sd.char_def, sd.unk_def)
     assert_batch_equal(vb.Tokenizer.new(raw).ignore_space(True).tokenize_batch(utf8=utf8, byte_offsets=off), tok_off, toks)
@@ -735,7 +725,8 @@ def test_row_longer_than_u16_follows_the_reference_truncation():
     the index wraps and the backtrack follows a different node than the one that gave the minimum — what the
     reference does is the specification, and the oracle restates it.  70 000 homographs of one surface also drive
     k_candidates' per-thread fallback (a postings list beyond the segment buffer's 255) and k_viterbi2's multi-pass
-    staging (rows longer than kPredCap)."""
+    staging (rows longer than kPredCap): pruned (viterbi_kernel 1), through the 64-bit-address lookup (0), and
+    through the unpruned twin that a batch holding a sentence of more than kPruneMaxChars characters takes."""
     n = 70000
     best = 69000  # the cheapest homograph sits beyond u16: 69000 as u16 = 3464
     rows = [f"a,1,1,{1000 if i != best else 10},h{i}" for i in range(n)] + ["b,1,1,5,B"]
@@ -746,7 +737,7 @@ def test_row_longer_than_u16_follows_the_reference_truncation():
     od = vo.OracleDictionary(lex, matrix, char_def, unk_def)
     utf8, off = vb.Tokenizer.pack(["ab", "a", "ba", "abab"])
     otok_off, otoks, _ = od.tokenize_batch(utf8, off)
-    for kernel in (1, 2, 0):
+    for kernel in (1, 0):
         tok = vb.Tokenizer.new(d)
         tok.set_option("viterbi_kernel", kernel)
         res = tok.tokenize_batch(utf8=utf8, byte_offsets=off)
@@ -754,3 +745,10 @@ def test_row_longer_than_u16_follows_the_reference_truncation():
     first = res.sentence_tokens(0)[0]
     assert first.feature() == f"h{best & 0xFFFF}"  # the truncated index, as in the reference
     assert res.sentence_tokens(1)[0].feature() == f"h{best & 0xFFFF}"  # insert_eos goes through the same u16 (lattice.rs:85-101)
+    utf8, off = vb.Tokenizer.pack(["ab", "a", "ba", "abab", "b" * 16001])
+    otok_off, otoks, _ = od.tokenize_batch(utf8, off)
+    assert_batch_equal(vb.Tokenizer.new(d).tokenize_batch(utf8=utf8, byte_offsets=off), otok_off, otoks)
+    for name, value in (("viterbi_kernel", 2), ("lanes_per_sentence", 8), ("sort_by_length", 0), ("dual_stream", 0)):
+        with pytest.raises(vb.VibratoError) as ei:  # retired options are unknown, not silently accepted
+            tok.set_option(name, value)
+        assert ei.value.kind == "InvalidArgument"

@@ -10,5 +10,5 @@ for spec in "$@"; do
       -Xptxas -v --expt-relaxed-constexpr $flags -c kernels.cu -o /tmp/kernels_$name.o 2> /tmp/kernels_$name.log
   /usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -shared -o ../libvibrato_b200_$name.so \
       host_dict.o device_blob.o capi.o engine.o multi_engine.o evaluate.o /tmp/kernels_$name.o -cudart static -ldl
-  echo "$name: $(grep -A2 'k_viterbi2ILi8ELi0ELb1ELb0' /tmp/kernels_$name.log | grep -E 'spill|Used' | tr -s ' ' | tr '\n' ' ')"
+  echo "$name: $(grep -A2 'k_viterbi2ILi0ELb1ELb0E' /tmp/kernels_$name.log | grep -E 'spill|Used' | tr -s ' ' | tr '\n' ' ')"
 done

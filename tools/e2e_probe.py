@@ -20,12 +20,9 @@ d = vb.SystemDictionaryBuilder.from_readers(sd.lex_csv, sd.matrix, sd.char_def, 
 tok = vb.Tokenizer.new(d)
 h_utf8 = torch.from_numpy(utf8).pin_memory().numpy()
 h_off = torch.from_numpy(off.astype(np.int64)).pin_memory().numpy().view(np.uint64)
-lanes_list = [int(x) for x in os.environ.get("VBT_PROBE_LANES", "8").split(",")]
 chunks = [int(x) for x in os.environ.get("VBT_PROBE_CHUNKS", "0,131072,262144,393216,524288").split(",")]
-for chunk, dual, lanes in [(c, 0, l) for l in lanes_list for c in chunks]:
+for chunk in chunks:
     tok.set_option("chunk_sentences", chunk)
-    tok.set_option("dual_stream", dual)
-    tok.set_option("lanes_per_sentence", lanes)
     for _ in range(2):
         r = tok.tokenize_batch(utf8=h_utf8, byte_offsets=h_off)
         del r
@@ -35,5 +32,5 @@ for chunk, dual, lanes in [(c, 0, l) for l in lanes_list for c in chunks]:
         ms = tok.last_stage_ms()
         del r
     wall = (time.perf_counter() - t) / 5 * 1e3
-    print(f"chunk={chunk:7d} dual={dual} lanes={lanes:2d} e2e wall={wall:7.2f}ms  stage sum={sum(ms.values()):7.2f}  viterbi={ms['viterbi']:6.2f} "
+    print(f"chunk={chunk:7d} e2e wall={wall:7.2f}ms  stage sum={sum(ms.values()):7.2f}  viterbi={ms['viterbi']:6.2f} "
           f"cand={ms['candidates']:5.2f} bt_write={ms['backtrack_write']:5.2f}", flush=True)

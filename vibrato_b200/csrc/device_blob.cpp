@@ -1,7 +1,6 @@
 #include "device_blob.hpp"
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <thread>
 
@@ -325,50 +324,38 @@ void pack_device_blob(const Dictionary& d, std::vector<uint8_t>& out) {
         for (uint32_t r = 0; r < nr; ++r) rc[rmap[r]] = d.dual_right_map[r];
         for (uint32_t l = 0; l < nl; ++l) lc[lmap[l]] = d.dual_left_map[l];
     } else if (!raw) {
-        // Stored transposed (mt[right][left]) unless VBT_MATRIX_LAYOUT=0: K3's lanes share a predecessor's
-        // right id and differ in the left ids of their candidates, so one request then reads one row.
-        const char* env = std::getenv("VBT_MATRIX_LAYOUT");
-        const bool transposed = !(env && env[0] == '0');
+        // Stored transposed (mt[right][left]): K3's lanes share a predecessor's right id and differ in the left ids
+        // of their candidates, so one request then reads one row.  Tiled so that the reads and the writes of a tile
+        // stay within a few lines; the two permutations scatter one side of the copy whatever the order, so the
+        // 240 M-entry unidic matrix is split over host threads (tiles of different left ids write different columns:
+        // no two threads touch the same element)
         int16_t* dm = reinterpret_cast<int16_t*>(out.data() + h.off_matrix);
         const int16_t* sm = d.matrix.data.data();
-        if (transposed) {
-            // tiled so that the reads and the writes of a tile stay within a few lines; the two permutations scatter
-            // one side of the copy whatever the order, so the 240 M-entry unidic matrix is split over host threads
-            // (tiles of different left ids write different columns: no two threads touch the same element)
-            constexpr uint32_t TB = 64;
-            const uint32_t n_tiles = (nl + TB - 1) / TB;
-            auto work = [&](uint32_t t0, uint32_t t1) {
-                for (uint32_t t = t0; t < t1; ++t) {
-                    const uint32_t l0 = t * TB, l1 = std::min(nl, l0 + TB);
-                    for (uint32_t r0 = 0; r0 < nr; r0 += TB) {
-                        const uint32_t r1 = std::min(nr, r0 + TB);
-                        for (uint32_t l = l0; l < l1; ++l) {
-                            const int16_t* src = sm + size_t(l) * nr;
-                            const size_t col = lmap[l];
-                            for (uint32_t r = r0; r < r1; ++r) dm[size_t(rmap[r]) * nl + col] = src[r];
-                        }
+        constexpr uint32_t TB = 64;
+        const uint32_t n_tiles = (nl + TB - 1) / TB;
+        auto work = [&](uint32_t t0, uint32_t t1) {
+            for (uint32_t t = t0; t < t1; ++t) {
+                const uint32_t l0 = t * TB, l1 = std::min(nl, l0 + TB);
+                for (uint32_t r0 = 0; r0 < nr; r0 += TB) {
+                    const uint32_t r1 = std::min(nr, r0 + TB);
+                    for (uint32_t l = l0; l < l1; ++l) {
+                        const int16_t* src = sm + size_t(l) * nr;
+                        const size_t col = lmap[l];
+                        for (uint32_t r = r0; r < r1; ++r) dm[size_t(rmap[r]) * nl + col] = src[r];
                     }
                 }
-            };
-            const uint32_t n_thr = size_t(nl) * nr < (1u << 22) ? 1u : std::min<uint32_t>(8, std::max<uint32_t>(1, std::thread::hardware_concurrency()));
-            if (n_thr <= 1) {
-                work(0, n_tiles);
-            } else {
-                std::vector<std::thread> th;
-                for (uint32_t i = 0; i < n_thr; ++i)
-                    th.emplace_back(work, uint32_t(uint64_t(n_tiles) * i / n_thr), uint32_t(uint64_t(n_tiles) * (i + 1) / n_thr));
-                for (auto& t : th) t.join();
             }
+        };
+        const uint32_t n_thr = size_t(nl) * nr < (1u << 22) ? 1u : std::min<uint32_t>(8, std::max<uint32_t>(1, std::thread::hardware_concurrency()));
+        if (n_thr <= 1) {
+            work(0, n_tiles);
         } else {
-            std::vector<uint16_t> rinv(nr);  // new right id -> old right id
-            for (uint32_t r = 0; r < nr; ++r) rinv[rmap[r]] = uint16_t(r);
-            for (uint32_t l = 0; l < nl; ++l) {
-                const int16_t* src = sm + size_t(l) * nr;
-                int16_t* dst = dm + size_t(lmap[l]) * nr;
-                for (uint32_t r = 0; r < nr; ++r) dst[r] = src[rinv[r]];
-            }
+            std::vector<std::thread> th;
+            for (uint32_t i = 0; i < n_thr; ++i)
+                th.emplace_back(work, uint32_t(uint64_t(n_tiles) * i / n_thr), uint32_t(uint64_t(n_tiles) * (i + 1) / n_thr));
+            for (auto& t : th) t.join();
         }
-        reinterpret_cast<BlobHeader*>(out.data())->matrix_transposed = transposed ? 1 : 0;
+        reinterpret_cast<BlobHeader*>(out.data())->matrix_transposed = 1;
     }
 }
 

@@ -60,7 +60,8 @@ struct BlobHeader {
     // these map an internal connection id to its column/row of it, and the raw sections hold the 8-lane term
     uint64_t off_right_conn, off_left_conn;  // u16[num_right] / u16[num_left]
     uint32_t m_num_right, m_num_left;
-    uint32_t matrix_transposed;  // connector_kind 0: 1 = matrix is i16[num_right][num_left] (see pack_device_blob)
+    uint32_t matrix_transposed;  // connector_kind 0: always 1, the matrix is i16[num_right][num_left]; the engine
+                                 // refuses an image with any other value
     uint32_t reserved1;
     // Output stage (tokenize/src/main.rs:83-127): per lexicon (0 system, 1 user, 2 unknown) the feature strings
     // (feat_off u32[n_words + 1] into feat bytes) and the word parameters in the dictionary's own connection

@@ -1,7 +1,6 @@
 // Device engine of the batched Viterbi tokenizer: HBM workspace + launch sequence (one stream).
 #include "engine.hpp"
 
-#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/iterator/transform_input_iterator.cuh>
 
@@ -84,40 +83,6 @@ struct CastU64 {
     __host__ __device__ unsigned long long operator()(uint32_t v) const { return v; }
 };
 
-__global__ void k_iota(uint32_t* v, uint32_t n) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) v[i] = i;
-}
-
-// Sentence order for K3: inside every tile of kOrderTile consecutive sentences, longest first.  K3 walks the
-// sentences of a warp (and block) in lockstep, so neighbours of similar length waste fewer steps, while a tile
-// stays small enough that the text and lattice rows of its sentences remain neighbours in memory (a global sort
-// by length was measured to lose more through scattered accesses than it gained).
-constexpr int kOrderTile = 256;
-__global__ void __launch_bounds__(kOrderTile) k_local_order(const uint32_t* __restrict__ n_slots, uint32_t n_sent,
-                                                          uint32_t* __restrict__ order) {
-    __shared__ unsigned long long key[kOrderTile];
-    const uint32_t i = blockIdx.x * kOrderTile + threadIdx.x;
-    // descending length, ties by index: key = (~len) << 32 | index, sorted ascending; padding sorts last
-    key[threadIdx.x] = i < n_sent ? ((unsigned long long)(~n_slots[i]) << 32) | i : ~0ull;
-    __syncthreads();
-    for (uint32_t k = 2; k <= kOrderTile; k <<= 1) {
-        for (uint32_t j = k >> 1; j > 0; j >>= 1) {
-            const uint32_t t = threadIdx.x, p = t ^ j;
-            if (p > t) {
-                const unsigned long long a = key[t], c = key[p];
-                const bool up = (t & k) == 0;
-                if ((a > c) == up) {
-                    key[t] = c;
-                    key[p] = a;
-                }
-            }
-            __syncthreads();
-        }
-    }
-    if (i < n_sent) order[i] = uint32_t(key[threadIdx.x]);  // the tile's valid entries come first
-}
-
 // ConnIdCounter totals += the counts of one finished attempt (see EngineImpl::connid_begin / connid_commit).
 __global__ void k_add_u64(unsigned long long* dst, const unsigned long long* src, size_t n) {
     size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -141,14 +106,12 @@ __global__ void k_add_value(unsigned long long* tok_off, uint32_t n_plus_1, unsi
     if (i < n_plus_1) tok_off[i] += base;
 }
 
-struct Workspace {  // every per-(chunk of a)-batch device array; two of them let consecutive chunks overlap
+struct Workspace {  // every per-(chunk of a)-batch device array
     DevBuf n_slots, slot_off, eos, n_tok, code_sys, code_usr, cinfo, groupable, byte_pos, info, info_ex, ends_cnt,
-        ends_meta, cand, ends_hot, ends_cold, scan_tmp, iota, sort_keys, order;
-    cudaStream_t stream = nullptr;
+        ends_meta, cand, ends_hot, ends_cold, scan_tmp;
     void release() {
         for (DevBuf* b : {&n_slots, &slot_off, &eos, &n_tok, &code_sys, &code_usr, &cinfo, &groupable, &byte_pos, &info,
-                          &info_ex, &ends_cnt, &ends_meta, &cand, &ends_hot, &ends_cold, &scan_tmp, &iota, &sort_keys,
-                          &order})
+                          &info_ex, &ends_cnt, &ends_meta, &cand, &ends_hot, &ends_cold, &scan_tmp})
             b->release();
     }
 };
@@ -184,8 +147,6 @@ class EngineImpl final : public Engine {
             o.h_ctrl = static_cast<Control*>(pinned_alloc(sizeof(Control)));
         }
         CK(cudaEventCreateWithFlags(&in_done_, cudaEventDisableTiming));
-        CK(cudaStreamCreateWithFlags(&aux_stream_, cudaStreamNonBlocking));
-        for (auto& e : base_ready_) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         tok_base_.ensure(8);
         BlobHeader h;
         if (host_blob) {
@@ -197,6 +158,8 @@ class EngineImpl final : public Engine {
             CK(cudaStreamSynchronize(stream_));
         }
         if (h.magic != kBlobMagic || h.total_bytes != n_bytes) throw Error(kInvalidArgument, "not a vibrato_b200 dictionary image");
+        if (h.connector_kind == 0 && h.matrix_transposed != 1)
+            throw Error(kInvalidArgument, "dictionary image: the connection matrix is not stored transposed");
         // k_viterbi2 addresses the connection matrix with a fixed high address word: the matrix must not cross a
         // 4 GiB boundary.  Where the allocation happens to straddle one, the image is placed again, shifted so that
         // the matrix starts on the boundary (at most one extra matrix of padding).
@@ -252,8 +215,8 @@ class EngineImpl final : public Engine {
         dv_.unk_ent = reinterpret_cast<const uint2*>(blob_ + h.off_unk_ent);
         dv_.matrix = reinterpret_cast<const int16_t*>(blob_ + h.off_matrix);
         dv_.num_right = h.num_right;
-        dv_.conn_stride_left = h.matrix_transposed ? 1 : h.num_right;
-        dv_.conn_stride_right = h.matrix_transposed ? h.num_left : 1;
+        dv_.conn_stride_left = 1;
+        dv_.conn_stride_right = h.num_left;
         dv_.connector_kind = h.connector_kind;
         for (int li = 0; li < 3; ++li) {
             dv_.feat_off[li] = reinterpret_cast<const uint32_t*>(blob_ + h.off_feat_off[li]);
@@ -321,10 +284,7 @@ class EngineImpl final : public Engine {
         cudaStreamDestroy(out_stream_);
         tok_base_.release();
         for (auto* b : {&blob_own_, &in_utf8_, &in_off_, &connid_, &connid_try_, &fmt_len_, &fmt_off_, &fmt_text_off_, &fmt_text_}) b->release();
-        for (auto& w : ws_) w.release();
-        cudaStreamSynchronize(aux_stream_);
-        cudaStreamDestroy(aux_stream_);
-        for (auto& e : base_ready_) cudaEventDestroy(e);
+        ws_.release();
         for (auto& r : pool_) {
             pinned_free(r->tok_off);
             pinned_free(r->tokens);
@@ -337,14 +297,7 @@ class EngineImpl final : public Engine {
 
     void set_counting(bool on) override { counting_ = on; }
     void set_option(const std::string& name, long long value) override {
-        if (name == "lanes_per_sentence") {
-            if (value != 4 && value != 8 && value != 16 && value != 32)
-                throw Error(kInvalidArgument, "lanes_per_sentence must be 4, 8, 16 or 32");
-            lanes_ = int(value);
-        } else if (name == "sort_by_length") {
-            if (value < 0 || value > 2) throw Error(kInvalidArgument, "sort_by_length must be 0 (off), 1 (whole batch) or 2 (tiles)");
-            order_mode_ = int(value);
-        } else if (name == "connid_counting") {
+        if (name == "connid_counting") {
             // Worker::init_connid_counter (worker.rs:77-83) when switched on; every batch tokenised
             // while it is on is followed by update_connid_counts (worker.rs:90-93)
             cudaStreamSynchronize(stream_);
@@ -364,8 +317,6 @@ class EngineImpl final : public Engine {
             if (value < 0 || value > 3) throw Error(kInvalidArgument, "output_mode must be 0 (off), 1 mecab, 2 wakati or 3 detail");
             if (value != 0 && tok_bytes_ != 24) throw Error(kInvalidArgument, "compact_tokens and output_mode exclude each other");
             output_mode_ = uint32_t(value);
-        } else if (name == "dual_stream") {
-            dual_stream_ = value != 0;
         } else if (name == "chunk_sentences") {
             if (value < 0 || value > 0x7FFFFFFF) throw Error(kInvalidArgument, "chunk_sentences out of range");
             chunk_sentences_ = uint32_t(value);  // 0 disables the chunked host pipeline
@@ -379,7 +330,7 @@ class EngineImpl final : public Engine {
             if (value < 1 || value > 1000) throw Error(kInvalidArgument, "chars_estimate_permille out of range");
             chars_per_byte_ = double(value) / 1000.0;
         } else if (name == "viterbi_kernel") {
-            if (value < 0 || value > 2) throw Error(kInvalidArgument, "viterbi_kernel must be 0, 1 or 2");
+            if (value < 0 || value > 1) throw Error(kInvalidArgument, "viterbi_kernel must be 0 or 1");
             viterbi_kernel_ = int(value);
         } else if (name == "counting") {
             counting_ = value != 0;
@@ -495,11 +446,7 @@ class EngineImpl final : public Engine {
                 max_chunk_bytes = std::max(max_chunk_bytes, off[bounds[c + 1]] - off[bounds[c]]);
                 max_chunk_sent = std::max(max_chunk_sent, bounds[c + 1] - bounds[c]);
             }
-            ws_[0].stream = stream_;
-            ws_[1].stream = aux_stream_;
-            const uint32_t n_ws = dual_stream_ ? 2 : 1;
-            for (uint32_t i = 0; i < n_ws; ++i)
-                ensure_workspace(ws_[i], max_chunk_sent, max_chunk_bytes);  // sized once: no cudaMalloc in the pipeline
+            ensure_workspace(ws_, max_chunk_sent, max_chunk_bytes);  // sized once: no cudaMalloc in the pipeline
             for (auto& o : out_) {
                 o.tok_off.ensure((size_t(max_chunk_sent) + 1) * 8, 1.25);
                 o.tokens.ensure(size_t(max_chunk_bytes) * 24 + 24, 1.25);
@@ -511,7 +458,6 @@ class EngineImpl final : public Engine {
             h2d(in_off_.p, off, (size_t(n_sent) + 1) * 8, stream_, off_pinned && off == byte_off);
             CK(cudaEventRecord(in_done_, stream_));
             CK(cudaStreamWaitEvent(in_stream_, in_done_, 0));
-            CK(cudaStreamWaitEvent(aux_stream_, in_done_, 0));
             std::memset(stage_ms_, 0, sizeof(stage_ms_));
             std::memset(counters_, 0, sizeof(counters_));
             launches_ = 0;
@@ -575,21 +521,15 @@ class EngineImpl final : public Engine {
             for (uint32_t c = 0; c < n_chunks; ++c) {
                 OutSlot& o = out_[c & 1];
                 uint32_t s0 = bounds[c], s1 = bounds[c + 1];
-                // "dual_stream": chunks alternate between two workspaces / compute streams so that the head
-                // of chunk c+1 can fill SMs left idle by the tail of chunk c (measured: no gain on B200 —
-                // the concurrent kernels contend for the same L1/L2 — hence off by default)
-                Workspace& w = ws_[dual_stream_ ? (c & 1) : 0];
-                CK(cudaStreamWaitEvent(w.stream, h2d_ev[c], 0));
-                if (c >= 2) CK(cudaStreamWaitEvent(w.stream, o.drained, 0));  // slot reused: its D2H must be done
-                enqueue(w, d_utf8, d_off + s0, s1 - s0, off[s1] - off[s0], o, tok_base_.as<unsigned long long>(),
-                        c >= 1 ? base_ready_[(c - 1) & 1] : nullptr, base_ready_[c & 1]);
+                CK(cudaStreamWaitEvent(stream_, h2d_ev[c], 0));
+                if (c >= 2) CK(cudaStreamWaitEvent(stream_, o.drained, 0));  // slot reused: its D2H must be done
+                enqueue(ws_, stream_, d_utf8, d_off + s0, s1 - s0, off[s1] - off[s0], o, tok_base_.as<unsigned long long>());
                 if (!utf8_pinned && c + 1 < n_chunks) issue_h2d(c + 1);
                 if (c >= 1) drain(c - 1);
             }
             drain(n_chunks - 1);
             CK(cudaStreamSynchronize(out_stream_));
             CK(cudaStreamSynchronize(in_stream_));
-            CK(cudaStreamSynchronize(aux_stream_));
             CK(cudaStreamSynchronize(stream_));
             if (bad_offsets) {
                 release(r);
@@ -787,9 +727,8 @@ class EngineImpl final : public Engine {
             cub::TransformInputIterator<unsigned long long, CastU64, const uint32_t*> it(fmt_len_.as<uint32_t>(), CastU64());
             size_t tmp = 0;
             CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp, it, fmt_off_.as<unsigned long long>(), n_tok + 1, stream_));
-            ws_[0].scan_tmp.ensure(tmp + 1024, 1.5);
-            ws_[0].stream = stream_;
-            exclusive_scan(ws_[0], it, fmt_off_.as<unsigned long long>(), n_tok + 1);
+            ws_.scan_tmp.ensure(tmp + 1024, 1.5);
+            exclusive_scan(ws_, it, fmt_off_.as<unsigned long long>(), n_tok + 1, stream_);
         }
         unsigned long long tok_bytes = 0;
         CK(cudaMemcpyAsync(&tok_bytes, fmt_off_.as<unsigned long long>() + n_tok, 8, cudaMemcpyDeviceToHost, stream_));
@@ -818,9 +757,9 @@ class EngineImpl final : public Engine {
     }
 
     template <typename In, typename Out>
-    void exclusive_scan(Workspace& w, In in, Out out, size_t n) {
+    void exclusive_scan(Workspace& w, In in, Out out, size_t n, cudaStream_t st) {
         size_t cap = w.scan_tmp.cap;  // sized by ensure_workspace
-        CK(cub::DeviceScan::ExclusiveSum(w.scan_tmp.p, cap, in, out, n, w.stream));
+        CK(cub::DeviceScan::ExclusiveSum(w.scan_tmp.p, cap, in, out, n, st));
     }
 
     // Sizes every workspace array for batches of up to n_sent sentences / n_bytes bytes (upper
@@ -831,11 +770,6 @@ class EngineImpl final : public Engine {
         w.slot_off.ensure(ns * 4, 1.25);
         w.eos.ensure(ns * 16, 1.25);
         w.n_tok.ensure(ns * 4, 1.25);
-        if (order_mode_ == 1) {
-            w.iota.ensure(ns * 4, 1.25);
-            w.sort_keys.ensure(ns * 4, 1.25);
-        }
-        if (order_mode_) w.order.ensure(ns * 4, 1.25);
         const size_t ms = size_t(n_bytes) + n_sent + 1;
         w.code_sys.ensure(ms * 4, 1.25);
         if (dv_.usr_table) w.code_usr.ensure(ms * 4, 1.25);
@@ -851,28 +785,21 @@ class EngineImpl final : public Engine {
         w.cand.ensure(want_cand * 16);
         w.ends_hot.ensure((want_cand + ns) * 8);
         w.ends_cold.ensure((want_cand + ns) * 16);
-        size_t tmp = 0;  // cub temp storage for the largest scan / sort of this size
-        cub::DeviceScan::ExclusiveSum(nullptr, tmp, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), ms, w.stream);
+        size_t tmp = 0;  // cub temp storage for the largest scan of this size
+        cub::DeviceScan::ExclusiveSum(nullptr, tmp, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), ms, stream_);
         w.scan_tmp.ensure(tmp + 1024, 1.5);
-        if (order_mode_ == 1) {
-            cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr),
-                                                      static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(ns), 0,
-                                                      32, w.stream);
-            w.scan_tmp.ensure(tmp + 1024, 1.5);
-        }
     }
 
     // One whole batch from device-resident input into out_[0]; synchronises, retries on pool overflow.
     void run_whole(const uint8_t* d_utf8, const unsigned long long* d_off, uint32_t n_sent, uint64_t n_bytes) {
         OutSlot& o = out_[0];
-        ws_[0].stream = stream_;
         batch_total_bytes_ = n_bytes;
         for (int attempt = 0;; ++attempt) {
-            ensure_workspace(ws_[0], n_sent, n_bytes);
+            ensure_workspace(ws_, n_sent, n_bytes);
             o.tok_off.ensure((size_t(n_sent) + 1) * 8, 1.25);
             o.tokens.ensure(size_t(n_bytes) * 24 + 24, 1.25);  // a token spans >= 1 character >= 1 byte
             connid_begin(stream_);
-            enqueue(ws_[0], d_utf8, d_off, n_sent, n_bytes, o, nullptr, nullptr, nullptr);
+            enqueue(ws_, stream_, d_utf8, d_off, n_sent, n_bytes, o, nullptr);
             CK(cudaEventSynchronize(o.done));
             CK(cudaGetLastError());
             if (o.h_ctrl->flags & kFlagBadOffsets)
@@ -901,11 +828,11 @@ class EngineImpl final : public Engine {
         if (counting_) std::memcpy(counters_, o.h_ctrl->counters, sizeof(counters_));
     }
 
-    // Queues the whole kernel sequence for one (chunk of a) batch on stream_; no host synchronisation.
-    // `tok_base` (device) makes the chunk's token offsets global and is advanced by its token count.
-    void enqueue(Workspace& w, const uint8_t* d_utf8, const unsigned long long* d_off, uint32_t n_sent, uint64_t n_bytes,
-                 OutSlot& o, unsigned long long* tok_base, cudaEvent_t base_wait, cudaEvent_t base_signal) {
-        cudaStream_t st = w.stream;
+    // Queues the whole kernel sequence for one (chunk of a) batch on `st`; no host synchronisation.
+    // `tok_base` (device) makes the chunk's token offsets global and is advanced by its token count; the chunks of a
+    // batch run on one stream, which orders these updates.
+    void enqueue(Workspace& w, cudaStream_t st, const uint8_t* d_utf8, const unsigned long long* d_off, uint32_t n_sent,
+                 uint64_t n_bytes, OutSlot& o, unsigned long long* tok_base) {
         // characters <= bytes is the hard bound; the per-character launches are sized from the ratio learned on
         // earlier batches (plus slack), and a batch that exceeds it flags itself and is re-run with the hard bound
         const uint32_t hard_slots = uint32_t(n_bytes + n_sent);
@@ -920,7 +847,6 @@ class EngineImpl final : public Engine {
         b.launch_slots = max_slots;
         b.n_slots = w.n_slots.as<uint32_t>();
         b.slot_off = w.slot_off.as<uint32_t>();
-        b.order = (order_mode_ && n_sent > 1) ? w.order.as<uint32_t>() : nullptr;
         b.eos = w.eos.as<uint4>();
         b.n_tok = w.n_tok.as<uint32_t>();
         b.tok_off = o.tok_off.as<unsigned long long>();
@@ -958,28 +884,15 @@ class EngineImpl final : public Engine {
             CK(cudaMemsetAsync(b.n_slots, 0, 4, st));
         }
         CK(cudaEventRecord(o.ev[1], st));
-        exclusive_scan(w, b.n_slots, b.slot_off, size_t(n_sent) + 1);
-        if (b.order && order_mode_ == 2) {
-            k_local_order<<<(n_sent + kOrderTile - 1) / kOrderTile, kOrderTile, 0, st>>>(b.n_slots, n_sent, w.order.as<uint32_t>());
-            ++o.launches;
-        } else if (b.order) {
-            // K3 walks several sentences per warp in lockstep: group sentences of similar length
-            // (longest first, which also trims the tail of the launch)
-            k_iota<<<(n_sent + 255) / 256, 256, 0, st>>>(w.iota.as<uint32_t>(), n_sent);
-            size_t cap = w.scan_tmp.cap;
-            CK(cub::DeviceRadixSort::SortPairsDescending(w.scan_tmp.p, cap, b.n_slots, w.sort_keys.as<uint32_t>(),
-                                                         w.iota.as<uint32_t>(), w.order.as<uint32_t>(), int(n_sent), 0, 32,
-                                                         st));
-            ++o.launches;
-        }
+        exclusive_scan(w, b.n_slots, b.slot_off, size_t(n_sent) + 1, st);
         CK(cudaEventRecord(o.ev[2], st));
         launch_decode(dv_, b, st);
         CK(cudaEventRecord(o.ev[3], st));
         launch_candidates(dv_, b, max_slots, st);
         CK(cudaEventRecord(o.ev[4], st));
-        exclusive_scan(w, b.ends_cnt, RowMetaOut{b.ends_meta}, size_t(max_slots) + 1);
+        exclusive_scan(w, b.ends_cnt, RowMetaOut{b.ends_meta}, size_t(max_slots) + 1, st);
         CK(cudaEventRecord(o.ev[5], st));
-        o.launches += launch_viterbi(dv_, b, lanes_, viterbi_kernel_, st);
+        o.launches += launch_viterbi(dv_, b, viterbi_kernel_, st);
         if (b.counters || b.lid_count) {
             launch_count_lattice(dv_, b, st);
             ++o.launches;
@@ -990,16 +903,14 @@ class EngineImpl final : public Engine {
         {
             cub::TransformInputIterator<unsigned long long, CastU64, const uint32_t*> it(b.n_tok, CastU64());
             if (n_sent == 0) CK(cudaMemsetAsync(b.n_tok, 0, 4, st));
-            exclusive_scan(w, it, b.tok_off, size_t(n_sent) + 1);
+            exclusive_scan(w, it, b.tok_off, size_t(n_sent) + 1, st);
         }
         CK(cudaEventRecord(o.ev[8], st));
         launch_backtrack_write(b, st);
         k_publish_totals<<<1, 1, 0, st>>>(b.slot_off, b.tok_off, n_sent, dc);
         if (tok_base) {
-            if (base_wait) CK(cudaStreamWaitEvent(st, base_wait, 0));  // the previous chunk (other stream) bumped it
             k_add_base<<<(n_sent + 256) / 256, 256, 0, st>>>(b.tok_off, n_sent + 1, tok_base);
             k_bump_base<<<1, 1, 0, st>>>(tok_base, dc);
-            if (base_signal) CK(cudaEventRecord(base_signal, st));
             o.launches += 2;
         }
         CK(cudaEventRecord(o.ev[9], st));
@@ -1035,20 +946,15 @@ class EngineImpl final : public Engine {
     bool connid_on_ = false;
     uint32_t num_left_ = 0, num_right_ = 0;
     std::vector<uint16_t> left_ids_, right_ids_;
-    Workspace ws_[2];
-    cudaStream_t aux_stream_ = nullptr;
-    cudaEvent_t base_ready_[2] = {nullptr, nullptr};
+    Workspace ws_;
     std::vector<HostResult*> pool_, pool_free_;
     std::vector<uint64_t> rebased_;
     double cand_per_byte_ = 4.0;
     double chars_per_byte_ = 1.0;  // learned; 1.0 = the hard bound (every byte a character)
     bool counting_ = false;
-    int order_mode_ = 0;  // K3's sentence order: 0 input order, 1 whole batch by length, 2 by length inside tiles
     uint32_t output_mode_ = 0;
     uint64_t batch_total_bytes_ = 0;  // size of the input buffer of the batch in flight (bounds check in K1a)
     DevBuf fmt_len_, fmt_off_, fmt_text_off_, fmt_text_;
-    bool dual_stream_ = false;
-    int lanes_ = 8;
     uint32_t tok_bytes_ = 24;
     int viterbi_kernel_ = 1;  // 1 = k_viterbi2 with pruning (kernels.cuh)
     float stage_ms_[kNumStages];

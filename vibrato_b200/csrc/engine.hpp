@@ -64,9 +64,8 @@ class Engine {
     virtual std::string describe() const = 0;  // JSON: devices, how the dictionary travelled, ...
 
     virtual void set_counting(bool on) = 0;
-    // Knobs: "lanes_per_sentence" (4/8/16/32), "sort_by_length" (0/1), "counting" (0/1), "chunk_sentences",
-    // "dual_stream", "connid_counting", "output_mode" (0 none, 1 mecab, 2 wakati, 3 detail: run_host also
-    // produces HostResult::text).
+    // Knobs: "counting" (0/1), "chunk_sentences", "connid_counting", "output_mode" (0 none, 1 mecab, 2 wakati,
+    // 3 detail: run_host also produces HostResult::text).
     virtual void set_option(const std::string& name, long long value) = 0;
     // Launch on a caller-owned CUDA stream (0 restores the engine's own stream).
     virtual void set_stream(uint64_t stream) = 0;

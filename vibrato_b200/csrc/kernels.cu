@@ -3,7 +3,7 @@
 //   K1a count_chars     warp / sentence   UTF-8 validation + character count
 //   K1b decode          warp / sentence   code points -> CharInfo, trie codes, c2b, groupable
 //   K2  candidates      thread / char     common-prefix walks (user, system) + unknown words
-//   K3  viterbi2        G lanes / sentence left-to-right min-plus DP over the lattice + EOS
+//   K3  viterbi2        8 lanes / sentence left-to-right min-plus DP over the lattice + EOS
 //       count_lattice   thread / sentence counted runs only: SURVEY.md §8(d) counters and connection-id counts,
 //                                         read off the finished lattice
 //   K4a backtrack_count thread / sentence length of the best path
@@ -17,15 +17,8 @@
 
 // A batch whose byte offsets k_count_chars refused is not touched by any later kernel: the sizes derived from
 // the offsets (slots, workspace bounds) cannot be trusted.
-#ifndef VBT_GUARD_OFFSETS
-#define VBT_GUARD_OFFSETS 1
-#endif
-#if VBT_GUARD_OFFSETS
 #define VBT_STAND_DOWN_IF_REJECTED(b) \
     if (*(b).flags & kFlagsStandDown) return
-#else
-#define VBT_STAND_DOWN_IF_REJECTED(b) (void)0
-#endif
 
 namespace vbt {
 
@@ -89,9 +82,7 @@ __device__ __forceinline__ uint32_t utf8_len_checked(const uint8_t* p, unsigned 
 
 // Sentences per warp of the warp-per-sentence kernels (K1a, K1b, K4b): a warp walks a few consecutive sentences so
 // that the grid has fewer, longer-lived blocks.
-#ifndef VBT_SENT_PER_WARP
-#define VBT_SENT_PER_WARP 4
-#endif
+constexpr uint32_t kSentPerWarp = 4;
 
 __device__ __forceinline__ void count_chars_one(const Batch& b, uint32_t s, uint32_t lane) {
     unsigned long long bo = b.byte_off[s], len = b.byte_off[s + 1] - bo;
@@ -136,8 +127,8 @@ __global__ void __launch_bounds__(256) k_count_chars(Batch b) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t lane = threadIdx.x & 31;
 #pragma unroll 1
-    for (uint32_t r = 0; r < VBT_SENT_PER_WARP; ++r) {
-        const uint32_t s = w * VBT_SENT_PER_WARP + r;
+    for (uint32_t r = 0; r < kSentPerWarp; ++r) {
+        const uint32_t s = w * kSentPerWarp + r;
         if (s >= b.n_sent) return;
         count_chars_one(b, s, lane);
     }
@@ -218,8 +209,8 @@ __global__ void __launch_bounds__(256) k_decode(DictView d, Batch b) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t lane = threadIdx.x & 31;
 #pragma unroll 1
-    for (uint32_t r = 0; r < VBT_SENT_PER_WARP; ++r) {
-        const uint32_t s = w * VBT_SENT_PER_WARP + r;
+    for (uint32_t r = 0; r < kSentPerWarp; ++r) {
+        const uint32_t s = w * kSentPerWarp + r;
         if (s >= b.n_sent) return;
         decode_one(d, b, s, lane);
         __syncwarp();
@@ -354,7 +345,7 @@ __global__ void __launch_bounds__(256) k_candidates(DictView d, Batch b) {
     // A rejected batch (see VBT_STAND_DOWN_IF_REJECTED) leaves every thread out of range.  The flag word is read
     // next to the slot total instead of in front of it: with 256-thread blocks that live for one trie walk, a
     // dependent extra round trip at the top costs 8 % of this kernel (profiles/r01e_k3_variants_ab.md).
-    const uint32_t batch_flags = VBT_GUARD_OFFSETS ? *b.flags : 0u;
+    const uint32_t batch_flags = *b.flags;
     const uint32_t total_slots = b.slot_off[b.n_sent];
     if (slot == 0 && total_slots > b.launch_slots) atomicOr(b.flags, kFlagSlotsOverflow);
     const bool in_range = slot < total_slots && !(batch_flags & kFlagBadOffsets);
@@ -489,7 +480,7 @@ __global__ void __launch_bounds__(256) k_candidates(DictView d, Batch b) {
 // K3: Tokenizer::build_lattice_inner (tokenizer.rs:94-139) + Lattice::insert_node / search_min_node /
 //     insert_eos (lattice.rs:85-151).
 //
-// G lanes per sentence (32 / G sentences per warp, walking their start positions in lockstep, one position after
+// 8 lanes per sentence (4 sentences per warp, walking their start positions in lockstep, one position after
 // the other), built around what the r01f profile showed to be the limits — warp-instruction issue and the LSU data
 // pipe of the L1 (shuffles, spills and gathers all queue there):
 //   * per position the candidates of the warp's sentences are dealt to the 32 lanes as one pool, lane = candidate;
@@ -567,15 +558,12 @@ struct ConnRow<2> {  // DualConnector::cost (dual_connector.rs:269-280): reduced
     }
 };
 
-#ifndef VBT_K3V2_WARPS
-#define VBT_K3V2_WARPS 4  // warps per block of k_viterbi2
-#endif
-#ifndef VBT_K3V2_MIN_BLOCKS
-#define VBT_K3V2_MIN_BLOCKS (64 / VBT_K3V2_WARPS)  // 64 warps per SM = 32 registers per thread
-#endif
-#ifndef VBT_K3V2_PF_DIST
-#define VBT_K3V2_PF_DIST 8
-#endif
+// k_viterbi2's shape.  Other block sizes and prefetch distances measured no different (profiles/r02_k3_variants_ab.md).
+constexpr int kV2Lanes = 8;                        // lanes of a warp per sentence
+constexpr uint32_t kV2SentPerWarp = 32 / kV2Lanes;
+constexpr int kV2Warps = 4;                        // warps per block
+constexpr int kV2MinBlocks = 64 / kV2Warps;        // 64 warps per SM = 32 registers per thread
+constexpr uint32_t kV2PrefetchDist = 8;            // candidate records ahead of the current position
 
 constexpr int kPredCap = 32;                             // predecessors staged per pass
 constexpr int32_t kPredSentinel = INT32_MAX - 70000;     // + any i16 stays below INT32_MAX and above every real best
@@ -672,27 +660,23 @@ struct ConnCol : ConnRow<CONN == 3 ? 0 : CONN> {
 // Shared-memory window of one warp of k_viterbi2: a staging row per sentence ({cost, right} of the predecessors, up
 // to kPredCap per pass plus padding to whole batches; the odd multiple of 32 bytes skews the rows across the banks),
 // and per sentence the descriptor of its current position {cand_ptr, slot, row offset, K} and its candidate count.
-template <int G>
 struct V2Shared {
-    static constexpr uint32_t SPW = 32 / G;
     static constexpr uint32_t kRowBytes = (kPredCap + 4) * 8;
-    int2 rows[SPW][kPredCap + 4];
-    uint4 desc[SPW];
+    int2 rows[kV2SentPerWarp][kPredCap + 4];
+    uint4 desc[kV2SentPerWarp];
     uint32_t cnt[8];
 };
 
-template <int G, int CONN, bool PRUNE, bool SPACE>
+template <int CONN, bool PRUNE, bool SPACE>
 __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b, const uint32_t sw /* shared-window address of this warp's V2Shared */) {
-    constexpr uint32_t SPW = 32 / G;  // sentences per warp
-    constexpr uint32_t kRowBytes = V2Shared<G>::kRowBytes;
-    constexpr uint32_t kDescOff = SPW * kRowBytes, kCntOff = kDescOff + SPW * 16;
+    constexpr uint32_t kRowBytes = V2Shared::kRowBytes;
+    constexpr uint32_t kDescOff = kV2SentPerWarp * kRowBytes, kCntOff = kDescOff + kV2SentPerWarp * 16;
     const uint32_t lane = threadIdx.x & 31;
-    const uint32_t gl = lane % G, sub = lane / G;
-    const uint32_t sidx = ((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * SPW + sub;
+    const uint32_t gl = lane % kV2Lanes, sub = lane / kV2Lanes;
+    const uint32_t s = ((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * kV2SentPerWarp + sub;
 
     uint32_t slot = 0, slot_end = 0;
-    if (sidx < b.n_sent) {
-        const uint32_t s = b.order ? b.order[sidx] : sidx;
+    if (s < b.n_sent) {
         slot = b.slot_off[s];
         slot_end = b.slot_off[s + 1] - 1;
         if (gl == 0) {
@@ -734,11 +718,9 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
         }
         if (ncand == 0) K = 0;
         const uint32_t max_k = __reduce_max_sync(kFull, K);
-#if VBT_K3V2_PF_DIST
         // K2 hands out the candidate pool in position order: pull the line of the positions ahead towards L1
-        if (ncand && gl == 0 && cptr + ncand + VBT_K3V2_PF_DIST < b.cand_cap)
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(b.cand + cptr + ncand + VBT_K3V2_PF_DIST));
-#endif
+        if (ncand && gl == 0 && cptr + ncand + kV2PrefetchDist < b.cand_cap)
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(b.cand + cptr + ncand + kV2PrefetchDist));
         // The candidates of the warp's sentences are dealt to the 32 lanes as ONE pool (sentence after sentence):
         // a position with 3 candidates next to one with 13 fills half a warp, not two rounds of 8-lane groups.
         // Every group publishes its position; a lane then finds which sentence its pool index falls into.
@@ -759,7 +741,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
             const uint32_t n_stage = (max_k + 1u) & ~1u;
             const uint32_t own = sw + sub * kRowBytes;
 #pragma unroll 1
-            for (uint32_t k = gl; k < n_stage; k += G) {
+            for (uint32_t k = gl; k < n_stage; k += kV2Lanes) {
                 if (k < K)
                     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(own + k * 8u), "l"(b.ends_hot + eo + k) : "memory");
                 else
@@ -774,7 +756,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
             {
                 bool adv = true;
 #pragma unroll
-                for (uint32_t i = 0; i + 1 < SPW; ++i) {
+                for (uint32_t i = 0; i + 1 < kV2SentPerWarp; ++i) {
                     uint32_t c;
                     asm volatile("ld.shared.b32 %0, [%1];" : "=r"(c) : "r"(sw + kCntOff + i * 4u));
                     adv = adv && q >= before + c;
@@ -813,7 +795,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
                     __syncwarp();
                     const uint32_t own = sw + sub * kRowBytes;
 #pragma unroll 1
-                    for (uint32_t k = gl; k < n_stage; k += G) {
+                    for (uint32_t k = gl; k < n_stage; k += kV2Lanes) {
                         int2 pr = make_int2(kPredSentinel, 0);
                         if (k0 + k < K) pr = b.ends_hot[eo + k0 + k];
                         asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(own + k * 8u), "r"(pr.x), "r"(pr.y) : "memory");
@@ -848,8 +830,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
 
     // Lattice::insert_eos (lattice.rs:85-101): left_id 0, no word cost; lanes of the group = predecessors
     {
-        const bool has_sentence = sidx < b.n_sent;
-        const uint32_t s = has_sentence ? (b.order ? b.order[sidx] : sidx) : 0;
+        const bool has_sentence = s < b.n_sent;
         const uint32_t base = has_sentence ? b.slot_off[s] : 0;
         const uint32_t n = has_sentence ? b.slot_off[s + 1] - 1 - base : 0;
         const uint32_t eos_start = slot_end - base;  // n, or the start of the trailing space run
@@ -864,7 +845,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
         long long bestkey = LLONG_MAX;
         const ConnCol<CONN> conn_eos(d, 0);  // BOS_EOS_CONNECTION_ID (common.rs:18)
         const uint32_t max_k = __reduce_max_sync(kFull, K);
-        for (uint32_t k0 = 0; k0 < max_k; k0 += G) {
+        for (uint32_t k0 = 0; k0 < max_k; k0 += kV2Lanes) {
             long long key = LLONG_MAX;
             if (k0 + gl < K) {
                 int2 pr = b.ends_hot[eo + k0 + gl];
@@ -872,7 +853,7 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
                 key = (long long)(((unsigned long long)uint32_t(v) << 32) | (unsigned long long)(~(k0 + gl)));
             }
 #pragma unroll
-            for (int o = G / 2; o > 0; o >>= 1) key = min(key, __shfl_xor_sync(kFull, key, o, G));
+            for (int o = kV2Lanes / 2; o > 0; o >>= 1) key = min(key, __shfl_xor_sync(kFull, key, o, kV2Lanes));
             bestkey = min(bestkey, key);
         }
         if (n > 0 && gl == 0) {
@@ -883,17 +864,18 @@ __device__ __forceinline__ void viterbi2_sweep(const DictView& d, const Batch& b
     }
 }
 
-// PRUNE and its unpruned twin are separate kernels launched back to back (each keeps its own register allocation);
-// the one the batch does not call for — kFlagLongSentence decides, and only the device knows it — returns at once.
+// CONN 0: PRUNE and its unpruned twin are separate kernels launched back to back (each keeps its own register
+// allocation); the one the batch does not call for — kFlagLongSentence decides, and only the device knows it —
+// returns at once.  CONN 1-3 never prune.
 // SPACE = the tokenizer ignores spaces: only then can a position carry a skip or the trailing flag.
-template <int G, int CONN, bool PRUNE, bool SPACE, bool TWIN>
-__global__ void __launch_bounds__(32 * VBT_K3V2_WARPS, CONN == 0 ? VBT_K3V2_MIN_BLOCKS : (32 / VBT_K3V2_WARPS)) k_viterbi2(DictView d, Batch b) {
+template <int CONN, bool PRUNE, bool SPACE>
+__global__ void __launch_bounds__(32 * kV2Warps, CONN == 0 ? kV2MinBlocks : (32 / kV2Warps)) k_viterbi2(DictView d, Batch b) {
     const uint32_t batch_flags = *b.flags;
     if (batch_flags & kFlagsStandDown) return;
-    if (TWIN && PRUNE == ((batch_flags & kFlagLongSentence) != 0)) return;
-    __shared__ __align__(16) V2Shared<G> s_warp[VBT_K3V2_WARPS];
+    if (CONN == 0 && PRUNE == ((batch_flags & kFlagLongSentence) != 0)) return;
+    __shared__ __align__(16) V2Shared s_warp[kV2Warps];
     const uint32_t sp = uint32_t(__cvta_generic_to_shared(&s_warp[threadIdx.x >> 5]));
-    viterbi2_sweep<G, CONN, PRUNE, SPACE>(d, b, sp);
+    viterbi2_sweep<CONN, PRUNE, SPACE>(d, b, sp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1018,8 +1000,8 @@ __global__ void __launch_bounds__(256) k_backtrack_write(Batch b) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t lane = threadIdx.x & 31;
 #pragma unroll 1
-    for (uint32_t r = 0; r < VBT_SENT_PER_WARP; ++r) {
-    const uint32_t s = w * VBT_SENT_PER_WARP + r;
+    for (uint32_t r = 0; r < kSentPerWarp; ++r) {
+    const uint32_t s = w * kSentPerWarp + r;
     if (s >= b.n_sent) return;
     const uint32_t base = b.slot_off[s];
     const unsigned long long t0 = b.tok_off[s];
@@ -1226,13 +1208,13 @@ void launch_format_write(const DictView& d, const FormatArgs& f, cudaStream_t st
 
 void launch_count_chars(const Batch& b, cudaStream_t st) {
     if (!b.n_sent) return;
-    uint32_t blocks = (b.n_sent + 8 * VBT_SENT_PER_WARP - 1) / (8 * VBT_SENT_PER_WARP);
+    uint32_t blocks = (b.n_sent + 8 * kSentPerWarp - 1) / (8 * kSentPerWarp);
     k_count_chars<<<blocks, 256, 0, st>>>(b);
 }
 
 void launch_decode(const DictView& d, const Batch& b, cudaStream_t st) {
     if (!b.n_sent) return;
-    uint32_t blocks = (b.n_sent + 8 * VBT_SENT_PER_WARP - 1) / (8 * VBT_SENT_PER_WARP);
+    uint32_t blocks = (b.n_sent + 8 * kSentPerWarp - 1) / (8 * kSentPerWarp);
     k_decode<<<blocks, 256, 0, st>>>(d, b);
 }
 
@@ -1242,44 +1224,32 @@ void launch_candidates(const DictView& d, const Batch& b, uint32_t max_slots, cu
     k_candidates<<<blocks, 256, 0, st>>>(d, b);
 }
 
-template <int G>
-static int launch_viterbi_g(const DictView& d, const Batch& b, int kernel, cudaStream_t st) {
+int launch_viterbi(const DictView& d, const Batch& b, int kernel, cudaStream_t st) {
+    if (!b.n_sent) return 0;
     const bool space = d.space_mask != 0;
-    const uint32_t per_block = VBT_K3V2_WARPS * (32 / G);
+    const uint32_t per_block = kV2Warps * kV2SentPerWarp;
     const uint32_t blocks = (b.n_sent + per_block - 1) / per_block;
-#define VBT_LAUNCH_V2(CONN, PRUNE, TWIN)                                                          \
-    do {                                                                                          \
-        if (space)                                                                                \
-            k_viterbi2<G, CONN, PRUNE, true, TWIN><<<blocks, 32 * VBT_K3V2_WARPS, 0, st>>>(d, b); \
-        else                                                                                      \
-            k_viterbi2<G, CONN, PRUNE, false, TWIN><<<blocks, 32 * VBT_K3V2_WARPS, 0, st>>>(d, b); \
+#define VBT_LAUNCH_V2(CONN, PRUNE)                                                  \
+    do {                                                                            \
+        if (space)                                                                  \
+            k_viterbi2<CONN, PRUNE, true><<<blocks, 32 * kV2Warps, 0, st>>>(d, b);  \
+        else                                                                        \
+            k_viterbi2<CONN, PRUNE, false><<<blocks, 32 * kV2Warps, 0, st>>>(d, b); \
     } while (0)
     int launched = 1;
     if (d.connector_kind == 1) {
-        VBT_LAUNCH_V2(1, false, false);
+        VBT_LAUNCH_V2(1, false);
     } else if (d.connector_kind == 2) {
-        VBT_LAUNCH_V2(2, false, false);
+        VBT_LAUNCH_V2(2, false);
     } else if (kernel == 0 || !d.matrix_window) {  // ConnCol<0> needs the matrix inside one 4 GiB window
-        VBT_LAUNCH_V2(3, false, false);
-    } else if (kernel == 1) {  // the pruned kernel and its twin for batches with very long sentences
-        VBT_LAUNCH_V2(0, true, true);
-        VBT_LAUNCH_V2(0, false, true);
+        VBT_LAUNCH_V2(3, false);
+    } else {  // the pruned kernel and its twin for batches with very long sentences
+        VBT_LAUNCH_V2(0, true);
+        VBT_LAUNCH_V2(0, false);
         launched = 2;
-    } else {
-        VBT_LAUNCH_V2(0, false, false);
     }
 #undef VBT_LAUNCH_V2
     return launched;
-}
-
-int launch_viterbi(const DictView& d, const Batch& b, int lanes_per_sentence, int kernel, cudaStream_t st) {
-    if (!b.n_sent) return 0;
-    switch (lanes_per_sentence) {
-        case 4: return launch_viterbi_g<4>(d, b, kernel, st);
-        case 8: return launch_viterbi_g<8>(d, b, kernel, st);
-        case 32: return launch_viterbi_g<32>(d, b, kernel, st);
-        default: return launch_viterbi_g<16>(d, b, kernel, st);
-    }
 }
 
 void launch_count_lattice(const DictView& d, const Batch& b, cudaStream_t st) {
@@ -1294,7 +1264,7 @@ void launch_backtrack_count(const Batch& b, cudaStream_t st) {
 
 void launch_backtrack_write(const Batch& b, cudaStream_t st) {
     if (!b.n_sent) return;
-    k_backtrack_write<<<(b.n_sent + 8 * VBT_SENT_PER_WARP - 1) / (8 * VBT_SENT_PER_WARP), 256, 0, st>>>(b);  // warps over sentences
+    k_backtrack_write<<<(b.n_sent + 8 * kSentPerWarp - 1) / (8 * kSentPerWarp), 256, 0, st>>>(b);  // warps over sentences
 }
 
 }  // namespace vbt

@@ -85,7 +85,6 @@ struct Batch {
     // per sentence
     uint32_t* n_slots;   // chars + 1 (scan input)
     uint32_t* slot_off;  // n_sent + 1
-    const uint32_t* order;  // sentence processing order of K3 (longest first), or nullptr
     uint4* eos;          // {best prev entry, start_node (sentence-relative), cost, 0}
     uint32_t* n_tok;
     unsigned long long* tok_off;  // n_sent + 1
@@ -138,11 +137,10 @@ void launch_format_write(const DictView& d, const FormatArgs& f, cudaStream_t st
 void launch_count_chars(const Batch& b, cudaStream_t st);
 void launch_decode(const DictView& d, const Batch& b, cudaStream_t st);
 void launch_candidates(const DictView& d, const Batch& b, uint32_t max_slots, cudaStream_t st);
-// K3 = k_viterbi2.  lanes_per_sentence in {4, 8, 16, 32}: how many lanes of a warp cooperate on one sentence.
-// kernel (matrix connector only): 1 = lower-bound pruning, with its unpruned twin for batches with very long
-// sentences; 2 = unpruned; 0 = the unpruned 64-bit-address lookup that a matrix crossing a 4 GiB address boundary
-// takes anyway.  Returns the number of kernels launched.
-int launch_viterbi(const DictView& d, const Batch& b, int lanes_per_sentence, int kernel, cudaStream_t st);
+// K3 = k_viterbi2.  kernel (matrix connector only): 1 = lower-bound pruning, with its unpruned twin for batches with
+// very long sentences; 0 = the unpruned 64-bit-address lookup that a matrix crossing a 4 GiB address boundary takes
+// anyway.  Returns the number of kernels launched.
+int launch_viterbi(const DictView& d, const Batch& b, int kernel, cudaStream_t st);
 // Counted runs only (b.counters or b.lid_count): the SURVEY.md §8(d) counters M, T, P, W, walks, E, N and the
 // connection-id counts, read off the lattice K3 left.  Runs between K3 and launch_backtrack_count.
 void launch_count_lattice(const DictView& d, const Batch& b, cudaStream_t st);
